@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path, one rank per GPU
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port) on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + the last timed step's track rows as .npy files
 
 One "step" = one frame of every resident stream through the whole per-frame path
 (uint8 frame -> stem/forward -> DFL decode -> NMS -> Kalman track bank update).
@@ -61,7 +62,12 @@ def parse():
     ap.add_argument("--no-kernels", action="store_true", help="skip the stand-alone HBM-kernel measurements")
     ap.add_argument("--total-streams", type=int, default=256, help="streams of the strong-scaling record (sharded over the GPUs)")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling record")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the track rows and counts of the last timed step (rank 0) as float64 .npy files to DIR")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 def peaks():
@@ -70,6 +76,37 @@ def peaks():
         d = json.load(open(p))
         return {"hbm": d["hbm_gbs"], "tc_burst": d["bf16_tflops"], "tc_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]), "src": "measured"}
     return {"hbm": 6650.0, "tc_burst": 1590.0, "tc_sustained": 1400.0, "src": "fallback"}
+
+
+I32_COLS = [0, 6, 7, 8, 9, 10, 11, 12, 16]     # columns of a track row that hold int32 bit patterns (include/b2dt.h)
+SLOT_COL = 19                                  # the bank's slot index of the track: implementation-defined
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, rows, counts):
+    """rows: CPU float32 [S][MAX_TRACKS_OUT][20], counts: CPU int32 [S] -> out_dir/{tracks,track_counts,stream_ids}.npy, float64.
+    Each stream's reported rows are sorted by track id (the reference's list order; the bank's own row order is an
+    implementation detail), int32 columns are converted to their values, the slot column (equally an implementation detail)
+    and unused rows are zero.  Streams beyond the
+    DUMP_BYTES budget are left out by a fixed-seed sample; stream_ids names the streams kept."""
+    import numpy as np
+
+    rows, counts = rows.numpy(), counts.numpy()
+    S = rows.shape[0]
+    assert int(counts.max()) <= rows.shape[1], "a stream reported more tracks than the result block holds"
+    k = min(S, DUMP_BYTES // (rows[0].size * 8 + 16))
+    ids = np.arange(S) if k == S else np.sort(np.random.default_rng(0).choice(S, k, replace=False))
+    out = np.zeros((k,) + rows.shape[1:], np.float64)
+    for j, s in enumerate(ids):
+        r = rows[s, :counts[s]]
+        v = r.astype(np.float64)
+        v[:, I32_COLS] = r.view(np.int32)[:, I32_COLS]
+        v[:, SLOT_COL] = 0
+        out[j, :len(v)] = v[np.argsort(v[:, 0], kind="stable")]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tracks.npy"), out)
+    np.save(os.path.join(out_dir, "track_counts.npy"), counts[ids].astype(np.float64))
+    np.save(os.path.join(out_dir, "stream_ids.npy"), ids.astype(np.float64))
 
 
 def make_frames(n_streams, n_frames, seed0=1000):
@@ -401,6 +438,9 @@ def run_b200(a):
         fwd_ms_insitu = sum(e0.elapsed_time(e1) for e0, e1 in pipe.forward_events) / len(pipe.forward_events)
     pipe.forward_events = None
     launches = lib.b2_launch_count() - l0
+    # step_device returns views of the bank's result block: take the last timed step's copy before the host-facing steps
+    # below overwrite it
+    last_out = (pipe.bank.rows.cpu(), pipe.bank.counts.cpu()) if a.dump_outputs and rank == 0 else None
     clocks = sampler.stop() if sampler else None
     value = S * world * a.steps / ms_dev * 1e3
 
@@ -536,6 +576,8 @@ def run_b200(a):
         dt = time.perf_counter() - t0
         line["cpu_baseline"] = {"value": n * k / dt, "unit": UNIT, "cores": cpu.cores, "kind": "port",
                                 "sample": f"{n} streams x {k} frames of the same workload (oracle port: numpy + ATen conv fp32, exact NMS, float64 tracker)"}
+    if last_out is not None:
+        dump_outputs(a.dump_outputs, *last_out)
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
     print(json.dumps(line), flush=True)

@@ -7,7 +7,8 @@ regenerate them anywhere; only the reference's OUTPUTS are stored (small .npz fi
 
 Files written:
   tracker_seq_f32.npz / tracker_seq_f64.npz   EnhancedMultiTargetTracker over a 260-frame multi-target
-                                              sequence (float32 resp. python-float detections)
+                                              sequence (float32 resp. python-float detections); the per-frame
+                                              Kalman states (x, P) in tracker_seq_{f32,f64}_states.npz
   tracker_kat.npz                             the 3-frame known-answer case of SURVEY.md 8c
   kf_ultra.npz                                KalmanFilterXYAH / XYWH initiate/predict/update/gating
   nms_cases.npz                               non_max_suppression, both branches (TorchNMS.nms / torchvision)
@@ -15,6 +16,7 @@ Files written:
   bytetrack.npz                               BYTETracker.update over a scripted 90-frame scene (two parameterisations) + linear_assignment cases
   overlay.npz                                 TrajectoryVisualizer.draw_tracks over a scripted 14-frame scene (annotated frames)
   predict_n_p2.npz / predict_s_p2.npz         YOLO(cfg).predict on 512x640 (and 500x640) frames + the NMS candidate lists
+  results_exports.npz                         Results.summary / save_txt / plot digests (golden_common.results_exports)
 """
 import contextlib
 import importlib.util
@@ -66,8 +68,10 @@ def gold_tracker():
             for tid, x, P, lf, il in st:
                 st_rows.append(np.r_[f, tid, x, P.reshape(-1), lf, float(il)])
         stats = trk.get_statistics()
+        # the per-frame Kalman states go to a file of their own: together with the rows they exceed 1 MB
+        np.savez_compressed(os.path.join(HERE, f"tracker_seq_{tag}_states.npz"), states=np.asarray(st_rows))
         np.savez_compressed(os.path.join(HERE, f"tracker_seq_{tag}.npz"), rows=rows, cols=np.array(cols), traj_len=tl,
-                            traj=tr.astype(np.float32), states=np.asarray(st_rows),
+                            traj=tr.astype(np.float32),
                             stats=np.array([stats[k] for k in ("total_tracks_created", "total_tracks_terminated",
                                                                "current_active_tracks", "long_term_predictions",
                                                                "successful_recoveries", "frame_count")]),
@@ -463,6 +467,15 @@ def gold_overlay():
     digests = np.array([hashlib.sha256(np.ascontiguousarray(o).tobytes()).hexdigest() for o in out])
     full = [0, 5, 8]                # whole frames for three of them (a failing digest can then be looked at), digests for all
     np.savez_compressed(os.path.join(HERE, "overlay.npz"), digests=digests, full_index=np.array(full), full=np.stack([out[i] for i in full]))
+
+
+def gold_results_exports():
+    """ultralytics/engine/results.py Results.summary / save_txt / plot over the fixed boxes of golden_common.results_exports."""
+    from golden_common import results_exports
+    from ultralytics.engine.results import Results
+
+    out = results_exports(lambda img, path, names, data: Results(img, path, names, boxes=torch.as_tensor(data)))
+    np.savez_compressed(os.path.join(HERE, "results_exports.npz"), **{k: np.array(v) for k, v in out.items()})
 
 
 if __name__ == "__main__":

@@ -269,3 +269,49 @@ def overlay_scene(n_frames=14, h=240, w=320):
         info = None if f == 2 else ({"frame_number": f, "state_changes": f // 4} if f % 2 else {"frame_number": f})
         frames.append((base.copy(), tracks, dets, info))
     return frames
+
+
+PLOT_KWARGS = ({}, {"conf": False}, {"labels": False}, {"line_width": 1}, {"line_width": 5}, {"color_mode": "instance"}, {"boxes": False})
+
+
+def results_exports(make):
+    """Results.summary / save_txt / plot over fixed boxes, with and without track ids (tests/golden/results_exports.npz):
+    ``make(img, path, names, data)`` builds a Results (the reference's or this package's).  Returns {key: str}: summaries as
+    JSON, save_txt files verbatim, plots as "shape dtype sha256" of their pixels -- boxes at the top / right edges, every
+    palette colour class, tracked and untracked rows, the plot switches, an image-scaled line width."""
+    import hashlib
+    import json
+    import os
+    import tempfile
+
+    def digest(a):
+        return f"{a.shape} {a.dtype} " + hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+    out = {}
+    img = np.zeros((96, 128, 3), np.uint8)
+    names = {0: "aircraft", 1: "bird"}
+    for data in (np.array([[10.5, 12.25, 30.0, 40.75, 0.912345, 0.0], [50.0, 20.0, 70.125, 44.0, 0.4, 1.0]], np.float32),
+                 np.array([[10.5, 12.25, 30.0, 40.75, 7.0, 0.912345, 0.0], [50.0, 20.0, 70.125, 44.0, 12.0, 0.4, 1.0]], np.float32)):
+        r, n = make(img, "a.jpg", names, data.copy()), data.shape[1]
+        out[f"summary_{n}"] = json.dumps(r.summary())
+        out[f"summary_normalized_{n}"] = json.dumps(r.summary(normalize=True, decimals=3))
+        for save_conf in (False, True):
+            with tempfile.TemporaryDirectory() as d:
+                p = os.path.join(d, "r.txt")
+                r.save_txt(p, save_conf=save_conf)
+                with open(p) as fh:
+                    out[f"txt_{n}_conf{int(save_conf)}"] = fh.read()
+    out["summary_empty"] = json.dumps(make(img, "a.jpg", names, np.zeros((0, 6), np.float32)).summary())
+    frame = np.random.default_rng(3).integers(0, 255, (240, 320, 3), dtype=np.uint8)
+    many = {c: f"class{c}" for c in range(24)}
+    xy = np.array([[4.2, 3.9, 60.0, 40.0], [250.5, 100.0, 318.0, 160.7], [100.0, 120.0, 101.0, 121.0], [-5.0, 200.0, 40.0, 260.0]], np.float32)
+    for tracked in (False, True):
+        rows = []
+        for c in range(24):
+            b = xy[c % 4] + np.float32(3 * (c // 4))
+            rows.append(np.concatenate([b, [100.0 + c] if tracked else [], [0.05 + 0.04 * c, float(c)]]))
+        r = make(frame, "a.jpg", many, np.array(rows, np.float32))
+        for j, kw in enumerate(PLOT_KWARGS):
+            out[f"plot_tracked{int(tracked)}_{j}"] = digest(r.plot(**kw))
+        out[f"plot_tracked{int(tracked)}_big"] = digest(r.plot(img=np.zeros((720, 1280, 3), np.uint8)))
+    return out

@@ -54,7 +54,7 @@ def _check_rows(rows, cols, g):
 
 def test_tracker_sequence_matches_reference():
     """260-frame multi-target sequence with misses, an occlusion burst and clutter (float32 detections)."""
-    g = np.load(os.path.join(G, "tracker_seq_f32.npz"))
+    g = dict(np.load(os.path.join(G, "tracker_seq_f32.npz")), states=np.load(os.path.join(G, "tracker_seq_f32_states.npz"))["states"])
     trk, outs, states = _run_gpu(int(g["seed"]), int(g["n_frames"]), g["params"], collect_state=True, n_targets=8)
     rows, cols, tl, tr = pack_tracks(outs)
     _check_rows(rows, cols, g)

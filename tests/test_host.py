@@ -26,7 +26,14 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), name
     assert lib.b2_version() >= 100
-    assert lib.b2_launch_count() == 0      # nothing was launched: no GPU here
+    import torch
+
+    if not torch.cuda.is_available():
+        assert lib.b2_launch_count() == 0      # nothing was launched: no GPU here
+    # loading the library launches nothing; checked in a fresh process, since GPU tests may have launched in this one
+    r = subprocess.run([sys.executable, "-c", f"import sys; sys.path.insert(0, {ROOT!r}); import b200dt; from b200dt import _lib; "
+                        "print(_lib.load(build_if_missing=False).b2_launch_count())"], capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.split() == ["0"], (r.stdout, r.stderr)
 
 
 def test_library_is_sm100a_with_tcgen05_and_tma():
@@ -276,12 +283,12 @@ def test_ultralytics_plugin_is_a_genuine_detection_predictor(tmp_path, monkeypat
     assert res[0].boxes.xyxy.cpu().numpy().dtype == np.float32
 
 
-def test_pt_checkpoint_loader_and_results_exports_match_reference(tmp_path, monkeypatch):
-    """N4: (a) weights.load_checkpoint reads the two checkpoint forms the reference writes (trainer: EMA half weights,
+def test_pt_checkpoint_loader_matches_reference(tmp_path, monkeypatch):
+    """N4: weights.load_checkpoint reads the two checkpoint forms the reference writes (trainer: EMA half weights,
     engine/trainer.py save_model; Model.save: `model` half weights) WITHOUT importing ultralytics -- same YAML dict, same
-    state_dict keys and values (fp16-widened), same names -- and the layer list resolves; (b) Results.summary / save_txt give the
-    reference's output for the same boxes, with and without track ids.  Build-container test (needs the reference checkout to
-    WRITE the checkpoint and to compare against)."""
+    state_dict keys and values (fp16-widened), same names -- and the layer list resolves.  Needs the reference checkout to
+    WRITE the checkpoints; where it is present, the stored exports of test_results_exports_match_reference are checked against
+    the reference's Results too."""
     import subprocess
     import sys
 
@@ -290,7 +297,6 @@ def test_pt_checkpoint_loader_and_results_exports_match_reference(tmp_path, monk
     import torch
 
     from b200dt import cfg, weights
-    from b200dt.predictor import Results
 
     gen = tmp_path / "gen.py"
     gen.write_text('''
@@ -311,7 +317,6 @@ torch.save({k: v for k, v in m.state_dict().items()}, sys.argv[3])
     p1, p2, p3 = tmp_path / "best.pt", tmp_path / "saved.pt", tmp_path / "sd.pt"
     env = dict(os.environ, YOLO_CONFIG_DIR=str(tmp_path))
     subprocess.run([sys.executable, str(gen), str(p1), str(p2), str(p3)], check=True, env=env, capture_output=True)
-    assert "ultralytics" not in sys.modules or True
     ref_sd = torch.load(p3, map_location="cpu")
     for p in (p1, p2):
         before = set(sys.modules)
@@ -325,42 +330,52 @@ torch.save({k: v for k, v in m.state_dict().items()}, sys.argv[3])
         spec = cfg.resolve(yd)
         assert spec["nc"] == 1 and spec["layers"][-1]["type"] == "Detect" and len(spec["layers"]) == len(yd["backbone"]) + len(yd["head"])
         assert [L["c_out"] for L in spec["layers"]] == [L["c_out"] for L in cfg.resolve("yolov8-small.yaml", nc=1)["layers"]]
-    # (b) exports
+    # the stored exports are the reference's
+    from golden_common import results_exports
+
     monkeypatch.setenv("YOLO_CONFIG_DIR", str(tmp_path))
     monkeypatch.syspath_prepend("/root/reference")
     from ultralytics.engine.results import Results as URes
 
-    img = np.zeros((96, 128, 3), np.uint8)
-    names = {0: "aircraft", 1: "bird"}
-    for data in (np.array([[10.5, 12.25, 30.0, 40.75, 0.912345, 0.0], [50.0, 20.0, 70.125, 44.0, 0.4, 1.0]], np.float32),
-                 np.array([[10.5, 12.25, 30.0, 40.75, 7.0, 0.912345, 0.0], [50.0, 20.0, 70.125, 44.0, 12.0, 0.4, 1.0]], np.float32)):
-        mine, ref = Results(img, "a.jpg", names, data.copy()), URes(img, "a.jpg", names, boxes=torch.as_tensor(data))
-        assert mine.summary() == ref.summary() and mine.summary(normalize=True, decimals=3) == ref.summary(normalize=True, decimals=3)
-        for save_conf in (False, True):
-            a, b = tmp_path / f"m{save_conf}{data.shape[1]}.txt", tmp_path / f"r{save_conf}{data.shape[1]}.txt"
-            mine.save_txt(a, save_conf=save_conf); ref.save_txt(b, save_conf=save_conf)
-            assert a.read_text() == b.read_text() and a.read_text().count("\n") == 2
-        assert mine.plot().shape == img.shape and mine.plot().any()
-    # plot(): the reference Annotator's pixels (OpenCV path) -- boxes at the top / right edges, every palette colour class,
-    # tracked and untracked rows, the switches
-    g = np.random.default_rng(3)
-    frame = g.integers(0, 255, (240, 320, 3), dtype=np.uint8)
-    many = {c: f"class{c}" for c in range(24)}
-    xy = np.array([[4.2, 3.9, 60.0, 40.0], [250.5, 100.0, 318.0, 160.7], [100.0, 120.0, 101.0, 121.0], [-5.0, 200.0, 40.0, 260.0]], np.float32)
-    for tracked in (False, True):
-        rows = []
-        for c in range(24):
-            b = xy[c % 4] + np.float32(3 * (c // 4))
-            rows.append(np.concatenate([b, [100.0 + c] if tracked else [], [0.05 + 0.04 * c, float(c)]]))
-        data = np.array(rows, np.float32)
-        mine, ref = Results(frame, "a.jpg", many, data.copy()), URes(frame, "a.jpg", many, boxes=torch.as_tensor(data))
-        for kw in ({}, {"conf": False}, {"labels": False}, {"line_width": 1}, {"line_width": 5}, {"color_mode": "instance"}, {"boxes": False}):
-            a, b = mine.plot(**kw), ref.plot(**kw)
-            assert a.dtype == np.uint8 and np.array_equal(a, b), (tracked, kw, int((a != b).any(-1).sum()))
-        assert np.array_equal(mine.orig_img, frame)
-        big = np.zeros((720, 1280, 3), np.uint8)                      # image-scaled line width 3, font scale 1
-        assert np.array_equal(mine.plot(img=big), ref.plot(img=big))
-    assert Results(img, "a.jpg", names, np.zeros((0, 6), np.float32)).summary() == []
+    _check_exports(results_exports(lambda img, path, names, data: URes(img, path, names, boxes=torch.as_tensor(data))))
+
+
+def _check_exports(got):
+    import json
+
+    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", "results_exports.npz"), allow_pickle=False)
+    assert set(got) == set(gold.files), set(got) ^ set(gold.files)
+    for k, v in got.items():
+        want = str(gold[k])
+        if k.startswith("summary"):
+            assert json.loads(v) == json.loads(want), (k, v, want)
+        else:
+            assert v == want, (k, v, want)
+
+
+def test_results_exports_match_reference():
+    """N4: Results.summary / save_txt / plot give the reference's output for the same boxes, with and without track ids
+    (golden/results_exports.npz; recipe in golden_common.results_exports): summaries and text files verbatim, plot() the
+    reference Annotator's pixels (OpenCV path) -- boxes at the top / right edges, every palette colour class, tracked and
+    untracked rows, the switches, an image-scaled line width (3, font scale 1 on 1280 x 720)."""
+    from golden_common import results_exports
+
+    from b200dt.predictor import Results
+
+    made = []
+
+    def make(img, path, names, data):
+        made.append((Results(img, path, names, data), img.copy()))
+        return made[-1][0]
+
+    got = results_exports(make)
+    _check_exports(got)
+    assert all(got[f"txt_{n}_conf{c}"].count("\n") == 2 for n in (6, 7) for c in (0, 1))
+    for r, img in made:
+        assert np.array_equal(r.orig_img, img)
+        p = r.plot()
+        assert p.dtype == np.uint8 and p.shape == img.shape and (p.any() or len(r) == 0)
+    assert Results(np.zeros((96, 128, 3), np.uint8), "a.jpg", {0: "aircraft"}, np.zeros((0, 6), np.float32)).summary() == []
 
 
 def _write_media(tmp_path, n_img=3, n_vid=7, hw=(96, 128)):
@@ -405,6 +420,16 @@ def test_file_loader_matches_reference(tmp_path, monkeypatch):
     assert [os.path.basename(p) for ps, _, _ in LoadImagesAndVideos(str(tmp_path / "list.txt")) for p in ps] == ["im0.png", "im2.png"]
     with pytest.raises(FileNotFoundError):
         LoadImagesAndVideos(str(tmp_path / "nope.mp4"))
+    # the reference loader's batches, stored: a batch never mixes the image list with a video, and a video is read by
+    # vid_stride grab() calls then retrieve() -- every frame at vid_stride=1, frames 1, 3, 5 of 7 at vid_stride=2
+    cap, seq = cv2.VideoCapture(clip), []
+    while (fr := cap.read())[0]:
+        seq.append(fr[1])
+    cap.release()
+    assert len(seq) == 7 and all(np.array_equal(im, seq[k]) for k, (_, im) in enumerate(flat[3:]))
+    s2 = [([os.path.basename(p) for p in ps], [i.copy() for i in im]) for ps, im, _ in LoadImagesAndVideos(str(tmp_path), batch=3, vid_stride=2)]
+    assert [n for n, _ in s2] == [["im0.png", "im1.png", "im2.png"], ["clip.avi"] * 3]
+    assert all(np.array_equal(im, seq[k]) for im, k in zip(s2[1][1], (1, 3, 5)))
     if os.path.isdir("/root/reference/ultralytics"):
         monkeypatch.setenv("YOLO_CONFIG_DIR", str(tmp_path / "cfg"))
         monkeypatch.syspath_prepend("/root/reference")

@@ -36,7 +36,7 @@ def _run_oracle_tracker(seed, n_frames, params, python_floats, **seq_kw):
 
 @pytest.mark.parametrize("tag,pyf", [("f32", False), ("f64", True)])
 def test_tracker_sequence_matches_reference(tag, pyf):
-    g = _load(f"tracker_seq_{tag}.npz")
+    g = dict(_load(f"tracker_seq_{tag}.npz"), states=_load(f"tracker_seq_{tag}_states.npz")["states"])
     trk, outs, states = _run_oracle_tracker(int(g["seed"]), int(g["n_frames"]), g["params"], pyf, n_targets=8)
     rows, cols, tl, tr = pack_tracks(outs)
     assert rows.shape == g["rows"].shape
