@@ -44,14 +44,15 @@ CONV_CASES = [
 ]
 
 
-TS_CASES = [c for c in CONV_CASES if c[5] == 3] + [
-    (2, 33, 19, 128, 64, 3, 1, True, True),       # 4 taps in tensor memory, 5 as SS MMAs from shared memory
-    (1, 48, 24, 80, 80, 3, 1, True, False),       # K segments 64 + 16, 6 resident taps
-    (2, 16, 32, 256, 80, 3, 1, True, False),      # 2 resident taps
-    (1, 31, 45, 32, 128, 3, 2, True, False),      # stride 2 through the transposed kernel (B2_CONV_TS=2)
-    (5, 8, 8, 64, 64, 3, 1, False, True),         # several images per tile, no activation
-    (3, 64, 48, 96, 64, 3, 2, True, False),       # stride 2 parity boxes, K segments 64 + 32, several images
-    (2, 34, 62, 16, 32, 3, 2, True, False),       # stride 2 parity boxes, ragged 17 x 31 output, 32-byte rows
+# the 3x3 shapes, run under both input-staging plans by test_conv_kernel_variants_match_oracle
+STAGING_CASES = [c for c in CONV_CASES if c[5] == 3] + [
+    (2, 33, 19, 128, 64, 3, 1, True, True),       # tap mode (map below the halo tile-efficiency cut), two images per tile, shortcut
+    (1, 48, 24, 80, 80, 3, 1, True, False),       # K segments 64 + 16; default: single halo box, two MMA warps
+    (2, 16, 32, 256, 80, 3, 1, True, False),      # three-box halo mode with streamed weights (too large to stay resident)
+    (1, 31, 45, 32, 128, 3, 2, True, False),      # stride 2, odd-sized input
+    (5, 8, 8, 64, 64, 3, 1, False, True),         # several images per tile, no activation, shortcut
+    (3, 64, 48, 96, 64, 3, 2, True, False),       # stride 2, K segments 64 + 32; default: parity boxes, two MMA warps
+    (2, 34, 62, 16, 32, 3, 2, True, False),       # stride 2 tap mode, ragged 17 x 31 output, several images per tile, 32-byte rows
 ]
 
 
@@ -106,11 +107,13 @@ def test_chained_conv_matches_oracle(case):
 
 
 @pytest.mark.parametrize("mode", ["0", "2"])
-@pytest.mark.parametrize("case", TS_CASES)
+@pytest.mark.parametrize("case", STAGING_CASES)
 def test_conv_kernel_variants_match_oracle(case, mode, monkeypatch):
-    """Both conv kernels on the same shapes: B2_CONV_TS=0 forces conv_tc_kernel (pixels x weights, SS MMAs),
-    B2_CONV_TS=2 forces conv_ts_kernel (weights in tensor memory, transposed accumulator) for every 3x3 conv."""
-    monkeypatch.setenv("B2_CONV_TS", mode)
+    """The 3x3 shapes under two input-staging plans of conv_tc_kernel.  mode = B2_CONV_HALO2: "2" is the default plan (one
+    (TW+2) x (TH+2) box per K chunk for resident-weight stride-1 layers, parity boxes for stride 2 where they fit); "0" turns
+    both single-box modes off (B2_CONV_S2BOX=0 too), so the same shapes stage one box per kw (halo 1) or one per filter tap."""
+    monkeypatch.setenv("B2_CONV_HALO2", mode)
+    monkeypatch.setenv("B2_CONV_S2BOX", "1" if mode == "2" else "0")
     test_conv_matches_oracle(case)
 
 

@@ -49,7 +49,7 @@ def main():
         for d in ls:
             w.writerow([d["id"], short(d["kernel"]), d["grid"], d["block"], round(d.get("time_us", 0), 2), int(d.get("dram_read_bytes", 0)),
                         int(d.get("dram_write_bytes", 0))])
-    conv = [d for d in fwd if "conv_tc_kernel" in d["kernel"] or "conv_ts_kernel" in d["kernel"]]
+    conv = [d for d in fwd if "conv_tc_kernel" in d["kernel"]]
     tot = sum(d.get("dram_read_bytes", 0) + d.get("dram_write_bytes", 0) for d in conv)
     shares = {}
     for d in fwd:

@@ -57,9 +57,6 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 // epilogue of conv_tc_kernel both use it, so the two paths give the same bits.
 constexpr float kLog2e = 1.4426950408889634f;
 __device__ __forceinline__ float dfl_exp(float f, float ml) { return ex2_ftz(fmaf(f, kLog2e, -ml)); }
-__device__ __forceinline__ float rcp_ftz(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-// SiLU(x) = x / (1 + 2^(-x log2 e)): two MUFU ops and three FP32 ops, flush-to-zero (no denormal fix-up code)
-__device__ __forceinline__ float silu_ex2(float x) { return x * rcp_ftz(1.0f + ex2_ftz(x * -1.4426950408889634f)); }
 // SiLU(x) = h + h tanh(h), h = x / 2: ONE MUFU op (tanh.approx.f32, max relative error 2^-11 on the tanh) and two FP32 ops.
 // Absolute error <= |h| * 2^-11 (reached on the negative lobe, |SiLU| <= 0.28 there): below the bf16 rounding of the stored
 // activation for every x > -1.5 and <= 1.2e-3 absolute beyond; the epilogues were MUFU / issue bound with the two-MUFU form.
@@ -203,45 +200,6 @@ __device__ __forceinline__ void tc_mma_bf16_if(uint32_t issue, uint32_t tmem_d, 
         "setp.ne.b32 q, %5, 0;\n\t"
         "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
         "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(issue) : "memory");
-}
-// D[tmem] (+)= A[tmem] * B[smem]^T: A = 128 lanes x 8 columns (16 bf16 along K, two per 32-bit column) of tensor memory
-__device__ __forceinline__ void tc_mma_ts_bf16_if(uint32_t issue, uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p, q;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "setp.ne.b32 q, %5, 0;\n\t"
-        "@q tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(issue) : "memory");
-}
-__device__ __forceinline__ void tc_mma_ts_bf16(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-}
-// registers -> 32 lanes x 8 consecutive 32-bit columns (thread t <-> lane base+t)
-__device__ __forceinline__ void tmem_st8(uint32_t addr, const uint4& a, const uint4& b) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 ::"r"(addr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// Same as tc_mma_bf16_if with the two descriptors given as 32-bit halves (packed inside the asm): the issue loop then
-// only does 32-bit uniform adds on the low words, the high words are loop constants.
-__device__ __forceinline__ void tc_mma_bf16_lohi_if(uint32_t issue, uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
-                                                    uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p, q;\n\t"
-        ".reg .b64 da, db;\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "setp.ne.b32 q, %7, 0;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "@q tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t"
-        "}" ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate), "r"(issue) : "memory");
 }
 __device__ __forceinline__ void tc_commit_if(uint32_t issue, uint64_t* bar) {
     asm volatile(

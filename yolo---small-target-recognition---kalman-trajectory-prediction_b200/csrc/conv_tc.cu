@@ -25,17 +25,6 @@
 //     C2f / SPPF / Concat / Detect become offset writes and offset reads.
 #include "common.cuh"
 
-// Experiment switches of the issue loops (tools/build_variant.sh): unrolled stride-2 stage, unrolled chained GEMM.  Both are OFF:
-// measured in one process on one box (tools/ab_chain.py), the unrolled forms issue fewer instructions per MMA but run SLOWER
-// (32->64 s2 chain 523 -> 586 us, DFL chain 488 -> 539 us): each tile then executes ~1000 straight-line instructions once
-// instead of a loop body that stays in the instruction cache, next to four other warp roles doing the same.
-#ifndef B2_S2_UNROLL
-#define B2_S2_UNROLL 0
-#endif
-#ifndef B2_CHAIN_UNROLL
-#define B2_CHAIN_UNROLL 0
-#endif
-
 #include <limits.h>
 
 #include <algorithm>
@@ -49,12 +38,6 @@ constexpr int kMaxNTile = 256;
 constexpr int kMaxAcc = 4;                         // accumulator stages in tensor memory
 constexpr int kMaxSeg = 4;                         // up to two sources (Concat folded into the conv) x two chunk widths
 constexpr int kMaxChainBlk = 6;                    // K blocks of a chained 1x1 conv (<= 384 channels)
-
-// transposed (TS) kernel: TMEM columns of one accumulator stage / of the weight region, K-elements the weight region holds
-constexpr uint32_t kTsAccCols = 128, kTsWeightCol = 256, kTsWeightK = 512;
-constexpr int kTsMmaWarps = 2, kTsDrainWarps = 8, kTsMathWarps = 8;
-constexpr int kTsThreads = 32 * (1 + kTsMmaWarps + kTsDrainWarps + kTsMathWarps);   // warp 0 TMA, 1..2 MMA, 3..10 drain, 11..18 math
-constexpr int kTsMaxSeg = 2;                      // single-source convs only: 64-channel chunks + one remainder segment
 
 // One K segment: `kchunks` chunks of `bk` channels starting at channel `c_off`.
 struct alignas(64) Seg {
@@ -70,7 +53,7 @@ struct alignas(64) Seg {
     uint32_t b_base;          // resident weights: offset of this segment's blocks inside the weight region
     uint32_t kh_step16;       // halo mode: (8 rows * row bytes) >> 4
     uint32_t desc_hi;         // high word of the shared-memory matrix descriptor (SBO, version, swizzle)
-    uint32_t desc_hi_w;       // the same for weight blocks (8-row pitch) where the pixel operand has another pitch (halo 2 / 3, conv_ts_kernel)
+    uint32_t desc_hi_w;       // the same for weight blocks (8-row pitch) where the pixel operand has another pitch (halo 2 / 3)
     uint32_t a_tx4[4];        // halo 3 (stride 2): bytes delivered by the box of parity view 0..3
     uint32_t desc_hi9;        // halo 3: pixel-operand descriptor high word for the 9-pixel-wide boxes (pw = 1)
 };
@@ -84,7 +67,7 @@ struct alignas(64) ConvParams {
     int n_tiles, n_tile, Cout;
     int Cin, ksize, stride, pad;
     int num_stages;
-    int halo;                 // 3x3 stride-1: 1 = one 18-row box per (kw, K chunk) serves the 3 kh taps (conv_tc_kernel);
+    int halo;                 // 3x3 stride-1: 1 = one 18-row box per (kw, K chunk) serves the 3 kh taps;
                               // 2 = one (TW+2) x (TH+2) box per K chunk serves all 9 taps by descriptor start row;
                               // 3 = 3x3 stride 2: one box per input parity (row, column) serves the 1 / 2 / 2 / 4 taps that read it
     int b_resident;           // 1: every weight block stays in shared memory for the lifetime of the CTA
@@ -100,22 +83,12 @@ struct alignas(64) ConvParams {
     int epi;                  // 0: bf16 channel-slice store; 1: DFL head (N = 64 -> 4 fp32 distances per pixel);
                               // 2: class head (N = nc -> fp32 {best logit, class} per pixel)   [Detect._inference fused]
     float* out_f32;           // epi 1: [pixels][4], epi 2: [pixels][2]
-    // ---- transposed "TS" variant (conv_ts_kernel): D^T[Cout, pixels] = W[Cout, K] * X[pixels, K]^T ----
-    int ts;                   // 1: launch conv_ts_kernel
-    int ts_res_taps;          // filter taps whose weights live in tensor memory; taps >= this come from shared memory (SS MMAs)
-    int tw_log2, th_log2;     // tile extents are powers of two
-    const __nv_bfloat16* w;   // [Cout][taps * Cin] weights (global), source of the tensor-memory copy
-    uint32_t stg_off;         // shared-memory offset of the fp32 staging tile(s) [128 pixels][cout16] of the transposing epilogue
-    int stg_bufs;             // 2: double buffered (one named barrier per tile), 1: single (two barriers)
-    uint32_t chunk_magic;     // ceil(2^32 / (cout16 / 16)): item -> pixel by a multiply-high
-    int ts_steps;             // pipeline stages one tile consumes
-    int mma_warps;            // conv_tc_kernel: 1 or 2 MMA-issuing warps (2: alternate tiles, two stage rings)
-    int epi_warps;            // conv_tc_kernel: 8 or 16 epilogue warps (16 only with two MMA warps, one CTA per SM)
-    int acc_stages;           // conv_tc_kernel: accumulator stages in tensor memory (2..4): tile t uses stage t % acc_stages
+    int mma_warps;            // 1 or 2 MMA-issuing warps (2: alternate tiles, two stage rings)
+    int epi_warps;            // 8 or 16 epilogue warps (16 only with two MMA warps, one CTA per SM)
+    int acc_stages;           // accumulator stages in tensor memory (2..4): tile t uses stage t % acc_stages
     uint32_t magic_nt, magic_tw, magic_th;   // ceil(2^32 / d) for d = n_tiles, tiles_w, tiles_h (0: d == 1) -- tile index -> coordinates
     int tma_lanes;            // halo 3: 4 = the producer issues four stage fills per instruction (lanes 0..3), 1 = one by one
     int halo3_k;              // halo 3: K chunks of all segments together (stage fills per parity view)
-    int dbg_skip_mma;         // B2_CONV_DEBUG=1: issue no MMAs (timing of the TMA / epilogue paths alone; results are garbage)
     // ---- chained 1x1 conv (conv_tc_kernel<.., CH = 1>): the activated bf16 tile of this conv never leaves the SM.  Half of the
     //      epilogue warps ("E1") write it into shared memory in the UMMA operand layout, the MMA warps run a second GEMM on it
     //      against the resident weights of the following 1x1 conv -- optionally together with K blocks loaded by TMA from the
@@ -349,36 +322,6 @@ __device__ __forceinline__ void ss_issue_taps(uint32_t leader, uint32_t d_addr, 
             accum = 1;
         }
     }
-}
-
-// One stage of a 3x3 stride-2 conv (halo 3), unrolled: the stage holds the (TW + PW) x (TH + PH) box of input parity (PH, PW); it
-// serves filter rows kh in {0, 2} (box rows 0 / 1) when PH else {1}, columns likewise.  row16 = one box row in descriptor units,
-// tb_lo = weight block (tap 0, this K chunk), tap_step = blocks between taps.
-template <int MPS, int PH, int PW>
-__device__ __forceinline__ void ss_issue_s2(uint32_t leader, uint32_t d_addr, uint32_t idesc, uint64_t hi_a, uint64_t hi_w, uint32_t a_lo,
-                                            uint32_t row16, uint32_t tb_lo, uint32_t tap_step, uint32_t& accum) {
-#pragma unroll
-    for (int a = 0; a <= PH; ++a) {
-#pragma unroll
-        for (int c = 0; c <= PW; ++c) {
-            const int kh = PH ? 2 * a : 1, kw = PW ? 2 * c : 1;
-            const uint32_t ta = a_lo + (uint32_t)(a * (8 + PW) + c) * row16;
-            const uint32_t tb = tb_lo + (uint32_t)(kh * 3 + kw) * tap_step;
-#pragma unroll
-            for (int j = 0; j < MPS; ++j) {
-                tc_mma_bf16_if(leader, d_addr, hi_a | (uint64_t)(ta + 2u * j), hi_w | (uint64_t)(tb + 2u * j), idesc, accum);
-                accum = 1;
-            }
-        }
-    }
-}
-template <int MPS>
-__device__ __forceinline__ void ss_issue_s2_g(int g, uint32_t leader, uint32_t d_addr, uint32_t idesc, uint64_t hi8, uint64_t hi9, uint64_t hi_w,
-                                              uint32_t a_lo, uint32_t row16, uint32_t tb_lo, uint32_t tap_step, uint32_t& accum) {
-    if (g == 0) ss_issue_s2<MPS, 0, 0>(leader, d_addr, idesc, hi8, hi_w, a_lo, row16, tb_lo, tap_step, accum);
-    else if (g == 1) ss_issue_s2<MPS, 0, 1>(leader, d_addr, idesc, hi9, hi_w, a_lo, row16, tb_lo, tap_step, accum);
-    else if (g == 2) ss_issue_s2<MPS, 1, 0>(leader, d_addr, idesc, hi8, hi_w, a_lo, row16, tb_lo, tap_step, accum);
-    else ss_issue_s2<MPS, 1, 1>(leader, d_addr, idesc, hi9, hi_w, a_lo, row16, tb_lo, tap_step, accum);
 }
 
 // MW: MMA-issuing warps.  1: warp 0 TMA, warp 1 MMA, warps 2..9 epilogue, up to two CTAs per SM.  2 (plans with ONE CTA per SM):
@@ -623,20 +566,6 @@ __global__ void __launch_bounds__(32 * (1 + MW + EW), MW == 1 ? 2 : 1) conv_tc_k
             const uint32_t d2 = tmem_base_u + p.c2_tmem_col + (uint32_t)(buf * p.c2_n);
             uint32_t accum2 = 0;
             const uint32_t buf_lo = smem_lo0 + p.c2_buf_off + (uint32_t)buf * p.c2_buf_bytes, w_lo0 = smem_lo0 + p.c2_wreg_off;
-#if B2_CHAIN_UNROLL
-#pragma unroll
-            for (int i = 0; i < kMaxChainBlk; ++i) {        // static indices: the per-block constants are read straight from the parameter bank
-                if (i < c2_nblk) {
-                    const uint32_t a_lo = (((buf_lo + p.c2_a_off[i]) >> 4) & 0x3FFFu) | (1u << 16);
-                    const uint32_t w_lo = (((w_lo0 + p.c2_w_off[i]) >> 4) & 0x3FFFu) | (1u << 16);
-                    const uint64_t hi = (uint64_t)p.c2_desc_hi[i] << 32;
-                    const int mps = p.c2_bk[i] >> 4;
-                    if (mps == 4) ss_issue_taps<4, 1>(leader, d2, idesc2, hi, a_lo, w_lo, 0u, accum2);
-                    else if (mps == 2) ss_issue_taps<2, 1>(leader, d2, idesc2, hi, a_lo, w_lo, 0u, accum2);
-                    else ss_issue_taps<1, 1>(leader, d2, idesc2, hi, a_lo, w_lo, 0u, accum2);
-                }
-            }
-#else
             for (int i = 0; i < c2_nblk; ++i) {
                 const uint32_t a_lo = (((buf_lo + p.c2_a_off[i]) >> 4) & 0x3FFFu) | (1u << 16);
                 const uint32_t w_lo = (((w_lo0 + p.c2_w_off[i]) >> 4) & 0x3FFFu) | (1u << 16);
@@ -646,7 +575,6 @@ __global__ void __launch_bounds__(32 * (1 + MW + EW), MW == 1 ? 2 : 1) conv_tc_k
                     accum2 = 1;
                 }
             }
-#endif
             tc_commit_if(leader, &t2_full[buf]);
             tc_commit_if(leader, &a2_empty[buf]);
         };
@@ -669,13 +597,6 @@ __global__ void __launch_bounds__(32 * (1 + MW + EW), MW == 1 ? 2 : 1) conv_tc_k
                         if (halo == 3) {
                             // stride 2: this stage holds the (TW + pw) x (TH + ph) box of input parity (ph, pw) = (g >> 1, g & 1); it
                             // serves taps kh in {0, 2} (box rows 0 / 1) or {1}, kw likewise (kh16 = one row); resident weights
-#if B2_S2_UNROLL
-                            const uint64_t hi9 = (uint64_t)sg_hi9[s] << 32;
-                            const uint32_t tb_lo = b_lo0 + b_base16 + (uint32_t)kc * b_blk16, tap_step = (uint32_t)kchunks * b_blk16;
-                            if (mma_per_step == 4) ss_issue_s2_g<4>(g, leader, d_addr, idesc, desc_hi_w, hi9, desc_hi_w, a_lo, kh16, tb_lo, tap_step, accum);
-                            else if (mma_per_step == 2) ss_issue_s2_g<2>(g, leader, d_addr, idesc, desc_hi_w, hi9, desc_hi_w, a_lo, kh16, tb_lo, tap_step, accum);
-                            else ss_issue_s2_g<1>(g, leader, d_addr, idesc, desc_hi_w, hi9, desc_hi_w, a_lo, kh16, tb_lo, tap_step, accum);
-#else
                             const int ph = g >> 1, pw = g & 1;
                             const uint64_t hi_a = pw ? (uint64_t)sg_hi9[s] << 32 : desc_hi_w;
                             const uint32_t row_pitch = (uint32_t)(8 + pw) * kh16;
@@ -691,7 +612,6 @@ __global__ void __launch_bounds__(32 * (1 + MW + EW), MW == 1 ? 2 : 1) conv_tc_k
                                     }
                                 }
                             }
-#endif
                         } else if (halo == 2) {
                             // one box, nine taps, resident weights: block (tap, kc)
                             const uint32_t tb_lo = b_lo0 + b_base16 + (uint32_t)kc * b_blk16, tb_step = (uint32_t)kchunks * b_blk16;
@@ -927,380 +847,6 @@ __global__ void __launch_bounds__(32 * (1 + MW + EW), MW == 1 ? 2 : 1) conv_tc_k
 }
 
 // ------------------------------------------------------------------------------------------------
-// Transposed variant for layers with few output channels (Cout <= 128).
-//
-// Measured on B200 (profiles/r01_mma_probe.txt): a tcgen05.mma whose two operands come from shared memory costs
-// ~102 cycles whatever N <= 128 is (each operand fetch has a ~51-cycle floor and they are serialised), i.e. an
-// M128 x N64 x K16 MMA runs at 31 % of the tensor pipe; with the A operand in TENSOR MEMORY the same instruction
-// at N = 128 runs at the pipe's floor (64 cycles).  So here the roles are swapped: A = the layer's weights, copied
-// once per CTA into tensor memory (lane = output channel, 2 bf16 of K per 32-bit column), B = the 128-pixel tile
-// staged by TMA exactly as in conv_tc_kernel (halo / tap modes, K segments, folded upsample+concat), and the
-// accumulator is D^T[lane = channel][column = pixel].  TMEM: 2 x 128 accumulator columns + 256 columns of weights
-// (512 K-elements); filter taps that do not fit are issued as SS MMAs on weights kept in shared memory.
-// Epilogue: thread = channel, columns = pixels; a warp's 32 lanes write 64 contiguous bytes of one NHWC pixel.
-// ------------------------------------------------------------------------------------------------
-
-// Drain helper: 32 accumulator columns (pixels pc0 .. pc0+31, pc0 % 4 == 0) of this thread's channel -> staging tile.
-// Staged element (pixel pc, channel c) lives in item it = pc * NCH + c / 16 (64 bytes); the item's four 16-byte quarters
-// are rotated by (it >> 1) & 3.  For NCH in {2, 4, 8} the rotation is periodic in the pixel index with period <= 4, so
-// every store is "base register + immediate": two instructions per element (FADD bias, STS).
-template <int NCH>
-__device__ __forceinline__ void ts_drain32(float* __restrict__ stg, int pc0, int nchunk_rt, const uint32_t (&v0)[16], const uint32_t (&v1)[16],
-                                           float bias, int c) {
-    const int cq = (c & 15) >> 2, cr = c & 3, cchunk = c >> 4;
-    if (NCH == 0) {
-        int it = pc0 * nchunk_rt + cchunk;
-#pragma unroll
-        for (int i = 0; i < 32; ++i, it += nchunk_rt)
-            stg[it * 16 + (((cq + (it >> 1)) & 3) << 2) + cr] = __uint_as_float(i < 16 ? v0[i & 15] : v1[i & 15]) + bias;
-    } else {
-        float* b[4];
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            // (it >> 1) & 3 for pixel pc0 + r (and every pixel congruent to it mod 4)
-            const int rot = NCH == 2 ? r : NCH == 4 ? ((cchunk >> 1) + 2 * (r & 1)) : (cchunk >> 1);
-            b[r] = stg + (pc0 * NCH + cchunk) * 16 + (((cq + rot) & 3) << 2) + cr;
-        }
-#pragma unroll
-        for (int i = 0; i < 32; ++i) b[i & 3][i * NCH * 16] = __uint_as_float(i < 16 ? v0[i & 15] : v1[i & 15]) + bias;
-    }
-}
-
-// All MMAs of one pipeline stage (TPG filter taps x MPS K-steps of 16), fully unrolled so that every descriptor is
-// one uniform add away from a stage base: at 64 cycles per MMA the issue warp is the critical resource.
-//   x_lo: descriptor low word of the stage's pixel box
-//   a_col: TMEM address of this stage's K chunk inside tap 0; tap_cols: TMEM columns per tap (Cin / 2)
-//   w_lo: smem descriptor low word of this stage's K chunk inside the first non-resident tap; w_tap16: (>>4) stride between taps
-template <int MPS, int TPG>
-__device__ __forceinline__ void ts_issue_stage(uint32_t leader, uint32_t d_addr, uint32_t idesc, uint64_t desc_hi, uint32_t x_lo,
-                                               uint32_t a_col, uint32_t tap_cols, uint32_t w_lo, uint32_t w_tap16, uint64_t desc_hi_w, int g,
-                                               int res_taps, uint32_t& accum) {
-#pragma unroll
-    for (int t = 0; t < TPG; ++t) {
-        const int tap = TPG == 9 ? t : g;
-        // halo stage: the tile's (TW+2) x (TH+2) pixel box; tap (kh, kw) starts kh * 10 + kw rows (of 32 * MPS bytes) in
-        const uint32_t tx_lo = x_lo + (uint32_t)(TPG == 9 ? ((t / 3) * 10 + (t % 3)) * 2 * MPS : 0);
-        if (tap < res_taps) {
-            const uint32_t ta = a_col + (uint32_t)tap * tap_cols;
-#pragma unroll
-            for (int j = 0; j < MPS; ++j) {
-                tc_mma_ts_bf16_if(leader, d_addr, ta + 8u * j, desc_hi | (uint64_t)(tx_lo + 2u * j), idesc, accum);
-                accum = 1;
-            }
-        } else {
-            const uint32_t tw = w_lo + (uint32_t)(tap - res_taps) * w_tap16;
-#pragma unroll
-            for (int j = 0; j < MPS; ++j) {
-                tc_mma_bf16_if(leader, d_addr, desc_hi_w | (uint64_t)(tw + 2u * j), desc_hi | (uint64_t)(tx_lo + 2u * j), idesc, accum);
-                accum = 1;
-            }
-        }
-    }
-}
-
-__global__ void __launch_bounds__(kTsThreads, 1) conv_ts_kernel(const __grid_constant__ ConvParams p) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t full_bar[kMaxStages];
-    __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
-    __shared__ __align__(8) uint64_t tfull_bar[2];
-    __shared__ __align__(8) uint64_t tempty_bar[2];
-    __shared__ __align__(8) uint64_t bres_bar;
-    __shared__ __align__(8) uint64_t stg_full_bar[2];
-    __shared__ __align__(8) uint64_t stg_empty_bar[2];
-    __shared__ uint32_t tmem_base_s;
-
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* smem_a = smem;                                           // pixel stages (B operand)
-    uint8_t* smem_b = smem + (size_t)p.num_stages * p.a_bytes;        // weights of the non-resident taps (SS A operand)
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const int taps = p.ksize * p.ksize;
-    const int res_taps = p.ts_res_taps;
-    const int nseg = p.nseg;
-
-    if (warp == 0 && lane == 0) {
-        for (int s = 0; s < nseg; ++s) {
-            tma_prefetch_desc(&p.seg[s].tmA[0]);
-            if (p.stride == 2) { tma_prefetch_desc(&p.seg[s].tmA[1]); tma_prefetch_desc(&p.seg[s].tmA[2]); tma_prefetch_desc(&p.seg[s].tmA[3]); }
-            tma_prefetch_desc(&p.seg[s].tmB);
-        }
-        for (int s = 0; s < p.num_stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-        const int n_drain = 2 * ((p.n_tile + 31) / 32);             // drain warps whose lane quadrant holds channels
-        for (int s = 0; s < 2; ++s) {
-            mbar_init(&tfull_bar[s], 1); mbar_init(&tempty_bar[s], 32 * n_drain);
-            mbar_init(&stg_full_bar[s], 32 * n_drain); mbar_init(&stg_empty_bar[s], 32 * kTsMathWarps);
-        }
-        mbar_init(&bres_bar, 1);
-        fence_mbar_init();
-    }
-    if (warp == 1) {
-        tmem_alloc(&tmem_base_s, 512);
-        tmem_relinquish();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_s;
-
-    // ---- weights of the resident taps -> tensor memory (warps 3..6 cover the four lane quadrants) ----
-    if (warp >= 3 && warp < 7) {
-        const int quad = warp & 3, c = quad * 32 + lane;
-        const int k_res = res_taps * p.Cin, k_total = taps * p.Cin;
-        const __nv_bfloat16* row = p.w + (size_t)c * k_total;
-        const uint32_t dst = tmem_base + kTsWeightCol + ((uint32_t)(quad * 32) << 16);
-        const bool have = c < p.Cout;
-        for (int k0 = 0; k0 < k_res; k0 += 16) {
-            uint4 v0 = make_uint4(0, 0, 0, 0), v1 = v0;
-            if (have) { v0 = __ldg(reinterpret_cast<const uint4*>(row + k0)); v1 = __ldg(reinterpret_cast<const uint4*>(row + k0 + 8)); }
-            tmem_st8(dst + (uint32_t)(k0 >> 1), v0, v1);
-        }
-        tmem_st_wait();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-
-    const int tiles_m = p.tiles_w * p.tiles_h * p.tiles_nb;
-    const int groups = p.halo ? 1 : taps;                 // halo (== 2 here): ONE (TW+2) x (TH+2) box per K chunk serves all nine taps
-
-    if (warp == 0) {
-        // ===================== TMA producer (pixel tiles; weights of the non-resident taps once) =====================
-        const bool leader = elect_one();
-        const int halo = p.halo, Cin = p.Cin, num_stages = p.num_stages;
-        const int ksz = p.ksize, pad = p.pad, stride = p.stride;
-        const int tiles_w = p.tiles_w, tiles_h = p.tiles_h, TW = p.TW, TH = p.TH, NB = p.NB;
-        const uint32_t a_bytes = p.a_bytes;
-        if (res_taps < taps && leader) {
-            mbar_expect_tx(&bres_bar, p.b_res_bytes);
-            for (int s = 0; s < nseg; ++s) {
-                const Seg& sg = p.seg[s];
-                for (int tap = res_taps; tap < taps; ++tap)
-                    for (int kc = 0; kc < sg.kchunks; ++kc)
-                        tma_load_2d(smem_b + sg.b_base + (size_t)((tap - res_taps) * sg.kchunks + kc) * sg.b_block_stride, &sg.tmB, &bres_bar,
-                                    tap * Cin + sg.c_off + kc * sg.bk, 0);
-            }
-        }
-        // two stage rings of num_stages / 2 slots: ring r holds the tiles issued by MMA warp r (a ring with two consumers
-        // would let one of them run a whole revolution ahead, which mbarrier phase parity cannot tell apart)
-        const int ring_stages = num_stages >> 1;
-        int rstage[2] = {0, 0}; uint32_t rphase[2] = {0, 0};
-        int ring = 0;
-        for (int tile = blockIdx.x; tile < tiles_m; tile += gridDim.x, ring ^= 1) {
-            int m_idx = tile;
-            const int w0 = (m_idx % tiles_w) * TW; m_idx /= tiles_w;
-            const int h0 = (m_idx % tiles_h) * TH;
-            const int n0 = (m_idx / tiles_h) * NB;
-            int stage = ring ? ring_stages + rstage[1] : rstage[0];
-            uint32_t phase = ring ? rphase[1] : rphase[0];
-            const int stage_lo = ring ? ring_stages : 0, stage_hi = stage_lo + ring_stages;
-            for (int g = 0; g < groups; ++g) {
-                int map = 0, cw, chh;
-                if (halo) {
-                    cw = w0 - 1; chh = h0 - 1;
-                } else {
-                    const int kh = g / ksz, kw = g % ksz;
-                    if (stride == 1) {
-                        cw = w0 + kw - pad; chh = h0 + kh - pad;
-                    } else {
-                        const int ih0 = kh - pad, iw0 = kw - pad;
-                        const int ph = ih0 & 1, pw = iw0 & 1;
-                        map = ph * 2 + pw;
-                        chh = h0 + (ih0 - ph) / 2; cw = w0 + (iw0 - pw) / 2;
-                    }
-                }
-                for (int s = 0; s < nseg; ++s) {
-                    const Seg& sg = p.seg[s];
-                    const int kchunks = sg.kchunks, bk = sg.bk;
-                    for (int kc = 0; kc < kchunks; ++kc) {
-                        mbar_wait(&empty_bar[stage], phase ^ 1);
-                        if (leader) {
-                            mbar_expect_tx(&full_bar[stage], sg.a_tx);
-                            if (sg.up == 2)
-                                tma_load_5d(smem_a + (size_t)stage * a_bytes, &sg.tmA[0], &full_bar[stage], sg.src_c + kc * bk, 0, cw >> 1, 0, n0 * sg.h_lo + (chh >> 1));
-                            else
-                                tma_load_4d(smem_a + (size_t)stage * a_bytes, &sg.tmA[map], &full_bar[stage], sg.src_c + kc * bk, cw, chh, n0);
-                        }
-                        __syncwarp();
-                        if (++stage == stage_hi) { stage = stage_lo; phase ^= 1; }
-                    }
-                }
-            }
-            if (ring) { rstage[1] = stage - ring_stages; rphase[1] = phase; } else { rstage[0] = stage; rphase[0] = phase; }
-        }
-    } else if (warp < 1 + kTsMmaWarps) {
-        // ===================== MMA issuers (warps 1, 2) =====================
-        // ncu showed the issuing warp busy all the time at ~150-190 cycles per MMA (latency chains through the uniform
-        // datapath) while the tensor pipe needs only 64: two warps issue alternate tiles, each owning one accumulator
-        // stage.  The producer fills the stage ring in tile order, so each warp skips the other warp's stages.
-        // Whole warp runs the loops with uniform control flow (one elected lane issues); single-source convs only
-        // (<= 2 K segments) keep the loop nest small enough for the instruction cache.
-        const int mw = warp - 1;
-        const uint32_t leader = elect_one() ? 1u : 0u;
-        // M = 128 lanes (channels, zero rows above Cout), N = 128 pixels
-        const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-        const uint32_t x_lo0 = ((smem_u32(smem_a) >> 4) & 0x3FFFu) | (1u << 16);
-        const uint32_t w_lo0 = ((smem_u32(smem_b) >> 4) & 0x3FFFu) | (1u << 16);
-        const uint32_t x_stage16 = p.a_bytes >> 4;
-        const uint32_t a_tm = tmem_base + kTsWeightCol;
-        const int halo = p.halo, num_stages = p.num_stages, Cin = p.Cin;
-        const int groups = halo ? 1 : taps;
-        int sg_kch[kTsMaxSeg], sg_mps[kTsMaxSeg];
-        uint32_t sg_hi[kTsMaxSeg], sg_hiw[kTsMaxSeg], sg_col0[kTsMaxSeg], sg_colstep[kTsMaxSeg], sg_blk16[kTsMaxSeg], sg_base16[kTsMaxSeg], sg_tap16[kTsMaxSeg];
-#pragma unroll
-        for (int s = 0; s < kTsMaxSeg; ++s) {
-            sg_kch[s] = s < nseg ? p.seg[s].kchunks : 0; sg_mps[s] = p.seg[s].bk >> 4;
-            sg_hi[s] = p.seg[s].desc_hi; sg_hiw[s] = p.seg[s].desc_hi_w;
-            sg_col0[s] = a_tm + (uint32_t)(p.seg[s].c_off >> 1); sg_colstep[s] = (uint32_t)(p.seg[s].bk >> 1);
-            sg_blk16[s] = p.seg[s].b_block_stride >> 4; sg_base16[s] = w_lo0 + (p.seg[s].b_base >> 4);
-            sg_tap16[s] = (uint32_t)p.seg[s].kchunks * (p.seg[s].b_block_stride >> 4);
-        }
-        const uint32_t tap_cols = (uint32_t)(Cin >> 1);
-        const int ring_stages = num_stages >> 1;
-        const int stage_lo = mw * ring_stages, stage_hi = stage_lo + ring_stages;       // this warp's stage ring
-        int stage = stage_lo; uint32_t phase = 0;
-        uint32_t acc_phase = 0;
-        const int skip_mma = p.dbg_skip_mma;
-        const int acc = mw;                                            // this warp's accumulator stage
-        const uint32_t d_addr = tmem_base + (uint32_t)acc * kTsAccCols;
-        if (res_taps < taps) { mbar_wait(&bres_bar, 0); tc_fence_after(); }
-        for (int tile = blockIdx.x + mw * gridDim.x; tile < tiles_m; tile += kTsMmaWarps * gridDim.x) {
-            mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-            tc_fence_after();
-            uint32_t accum = 0;
-            for (int g = 0; g < groups; ++g) {
-#pragma unroll
-                for (int s = 0; s < kTsMaxSeg; ++s) {
-                    const int kchunks = sg_kch[s], mps = sg_mps[s];
-                    const uint64_t desc_hi = (uint64_t)sg_hi[s] << 32, desc_hi_w = (uint64_t)sg_hiw[s] << 32;
-                    uint32_t a_col = sg_col0[s], w_lo = sg_base16[s];
-                    for (int kc = 0; kc < kchunks; ++kc) {
-                        mbar_wait(&full_bar[stage], phase);
-                        tc_fence_after();
-                        const uint32_t x_lo = x_lo0 + (uint32_t)stage * x_stage16;
-                        if (skip_mma) {
-                        } else if (halo) {
-                            if (mps == 4) ts_issue_stage<4, 9>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                            else if (mps == 2) ts_issue_stage<2, 9>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                            else ts_issue_stage<1, 9>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                        } else {
-                            if (mps == 4) ts_issue_stage<4, 1>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                            else if (mps == 2) ts_issue_stage<2, 1>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                            else ts_issue_stage<1, 1>(leader, d_addr, idesc, desc_hi, x_lo, a_col, tap_cols, w_lo, sg_tap16[s], desc_hi_w, g, res_taps, accum);
-                        }
-                        tc_commit_if(leader, &empty_bar[stage]);
-                        if (++stage == stage_hi) { stage = stage_lo; phase ^= 1; }
-                        a_col += sg_colstep[s]; w_lo += sg_blk16[s];
-                    }
-                }
-            }
-            tc_commit_if(leader, &tfull_bar[acc]);
-            acc_phase ^= 1;
-        }
-    } else if (warp < 1 + kTsMmaWarps + kTsDrainWarps) {
-        // ===================== drain warps (3..10, two per TMEM lane quadrant: 64 pixel columns each) =====================
-        // Accumulator D^T[lane = channel][column = pixel] (+ bias) -> fp32 staging tile in shared memory, laid out as
-        // items of 16 channels of one pixel (it = pixel * nchunk + chunk, 64 bytes).  The four 16-byte quarters of an item
-        // are rotated by (it >> 1) & 3 so that the math warps' 128-bit reads (consecutive lanes = consecutive items)
-        // hit eight different bank groups per quarter warp; a drain warp's 32 lanes write 128 contiguous bytes.
-        const int quad = warp & 3;
-        const int half = (warp - 1 - kTsMmaWarps) >> 2;
-        const int c = quad * 32 + lane;
-        const int cout16 = p.n_tile, nchunk = cout16 >> 4;
-        if (quad * 32 < cout16) {
-            const bool c_ok = c < cout16;
-            const float bias = c < p.Cout ? __ldg(p.bias + c) : 0.f;
-            float* const stg0 = reinterpret_cast<float*>(smem + p.stg_off);
-            const int stg_elems = 128 * cout16, nbufs = p.stg_bufs;
-            int acc = 0; uint32_t acc_phase = 0; int buf = 0; uint32_t buf_phase = 0;
-            for (int tile = blockIdx.x; tile < tiles_m; tile += gridDim.x) {
-                float* const stg = stg0 + buf * stg_elems;
-                mbar_wait(&stg_empty_bar[buf], buf_phase ^ 1);          // the math warps are done with this buffer
-                mbar_wait(&tfull_bar[acc], acc_phase);
-                tc_fence_after();
-                const uint32_t t_addr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)acc * kTsAccCols + (uint32_t)half * 64u;
-#pragma unroll 1
-                for (int jj = 0; jj < 4; jj += 2) {
-                    uint32_t v0[16], v1[16];
-                    tmem_ld16(t_addr + jj * 16, v0);
-                    tmem_ld16(t_addr + (jj + 1) * 16, v1);
-                    tmem_ld_wait();
-                    if (c_ok) {
-                        const int pc0 = half * 64 + jj * 16;
-                        if (nchunk == 4) ts_drain32<4>(stg, pc0, nchunk, v0, v1, bias, c);
-                        else if (nchunk == 2) ts_drain32<2>(stg, pc0, nchunk, v0, v1, bias, c);
-                        else if (nchunk == 8) ts_drain32<8>(stg, pc0, nchunk, v0, v1, bias, c);
-                        else ts_drain32<0>(stg, pc0, nchunk, v0, v1, bias, c);
-                    }
-                }
-                tc_fence_before();
-                mbar_arrive(&tempty_bar[acc]);                  // accumulator drained: the MMAs of the tile after next may start
-                mbar_arrive(&stg_full_bar[buf]);                // staged tile complete (release)
-                if (++buf == nbufs) { buf = 0; buf_phase ^= 1; }
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-            }
-        }
-    } else {
-        // ===================== math warps (11..18) =====================
-        // item = (pixel, 16-channel chunk) = 64 staged bytes -> the vectorised SiLU / residual / bf16 / 256-bit-store path
-        // of conv_tc_kernel; runs one tile behind the drain warps (double-buffered staging when it fits).
-        const int Cout = p.Cout, act = p.act, wide = p.wide;
-        const int cout16 = p.n_tile, nchunk = cout16 >> 4;
-        const int tiles_w = p.tiles_w, tiles_h = p.tiles_h, TW = p.TW, TH = p.TH, NB = p.NB;
-        const int lw = p.tw_log2, lh = p.th_log2;
-        const int Wo = p.Wo, Ho = p.Ho, Bn = p.B;
-        const int out_cstride = p.out_cstride, res_cstride = p.res_cstride;
-        __nv_bfloat16* const out0 = p.out + p.out_coff;
-        const __nv_bfloat16* const res0 = p.res ? p.res + p.res_coff : nullptr;
-        const float* const stg0 = reinterpret_cast<const float*>(smem + p.stg_off);
-        const int stg_elems = 128 * cout16, nbufs = p.stg_bufs;
-        const int et = threadIdx.x - 32 * (1 + kTsMmaWarps + kTsDrainWarps);      // 0..255
-        const int items = 128 * nchunk;
-        const uint32_t magic = p.chunk_magic;
-        int buf = 0; uint32_t buf_phase = 0;
-        for (int tile = blockIdx.x; tile < tiles_m; tile += gridDim.x) {
-            int m_idx = tile;
-            const int w0 = (m_idx % tiles_w) * TW; m_idx /= tiles_w;
-            const int h0 = (m_idx % tiles_h) * TH;
-            const int n0 = (m_idx / tiles_h) * NB;
-            const float* const stg = stg0 + buf * stg_elems;
-            mbar_wait(&stg_full_bar[buf], buf_phase);
-            for (int it = et; it < items; it += 32 * kTsMathWarps) {
-                const int pc = (int)__umulhi((uint32_t)it, magic);          // pixel (column of the accumulator)
-                const int ch = it - pc * nchunk;
-                const int w = w0 + (pc & (TW - 1)), h = h0 + ((pc >> lw) & (TH - 1)), n = n0 + (pc >> (lw + lh));
-                if ((w < Wo) && (h < Ho) && (n < Bn)) {
-                    const float4* src = reinterpret_cast<const float4*>(stg + (size_t)it * 16);
-                    const int rot = it >> 1;
-                    uint32_t v[16];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const float4 t4 = src[(q + rot) & 3];
-                        v[4 * q] = __float_as_uint(t4.x); v[4 * q + 1] = __float_as_uint(t4.y);
-                        v[4 * q + 2] = __float_as_uint(t4.z); v[4 * q + 3] = __float_as_uint(t4.w);
-                    }
-                    const size_t pix = ((size_t)n * Ho + h) * Wo + w;
-                    __nv_bfloat16* optr = out0 + pix * out_cstride + ch * 16;
-                    const __nv_bfloat16* rptr = res0 ? res0 + pix * res_cstride + ch * 16 : nullptr;
-                    const int nv = min(16, Cout - ch * 16);
-                    if (wide) epilogue_chunk<true, false>(v, nullptr, act, nv, optr, rptr);
-                    else epilogue_chunk<false, false>(v, nullptr, act, nv, optr, rptr);
-                }
-            }
-            mbar_arrive(&stg_empty_bar[buf]);
-            if (++buf == nbufs) { buf = 0; buf_phase ^= 1; }
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 512);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -1516,76 +1062,11 @@ int b2_conv_prepare_chain(void* storage, const B2ConvSrc* srcs, int nsrc, int B,
         }
     }
 
-    // ---- kernel variant: transposed "TS" kernel (weights in tensor memory) for MMA-issue-bound layers with Cout <= 128 ----
-    int ts_mode = 0;                                   // B2_CONV_TS: 0 never (default: conv_tc_kernel's single-box halo mode is faster today), 1 heuristic, 2 every 3x3 conv with Cout <= 128
-    if (const char* ev = getenv("B2_CONV_TS")) ts_mode = atoi(ev);
-    const int res_taps = Cin <= (int)kTsWeightK ? (taps < (int)kTsWeightK / Cin ? taps : (int)kTsWeightK / Cin) : 0;
-    p.ts = 0;
-    if (!chain && cout16 <= 128 && ksize == 3 && res_taps >= 1 && p.nseg <= kTsMaxSeg && p.halo != 3) {
-        if (ts_mode == 2) p.ts = 1;
-        else if (ts_mode == 1) p.ts = (p.halo && res_taps >= 3) ? 1 : 0;
-        size_t fb = 0;                                  // shared memory for the weights of the taps served by SS MMAs
-        for (int si = 0; si < p.nseg; ++si) fb += (size_t)(taps - res_taps) * p.seg[si].kchunks * up1k(128u * p.seg[si].bk * 2u);
-        const size_t a_ts = p.halo ? up1k((size_t)(p.TW + 2) * (p.TH + 2) * bk_max * 2) : (size_t)p.a_bytes;   // stage size in conv_ts_kernel
-        if (fb + (size_t)128 * cout16 * 4 + 4 * a_ts > 212 * 1024) p.ts = 0;
-    }
-    int ctas = 1, stages = 0;
-    if (p.ts && p.halo) {
-        // Measured: the TMA unit delivers one box row (<= 128 B) per ~7.6 cycles per SM, and the shared-memory operand of
-        // tcgen05.mma may start at ANY row with ANY 8-row-group pitch (the swizzle is a function of the absolute address,
-        // profiles/r01_shift_probe.txt).  So the tile's whole (TW+2) x (TH+2) halo box is loaded ONCE per K chunk
-        // (180 rows instead of 3 x 144) and tap (kh, kw) is the same tile at start row kh * (TW+2) + kw, pitch TW+2.
-        p.halo = 2;
-        a_rows = (p.TW + 2) * (p.TH + 2);
-        p.a_bytes = (uint32_t)up1k((size_t)a_rows * bk_max * 2);
-    }
-    if (p.ts) {
-        p.n_tiles = 1; p.n_tile = cout16; p.ts_res_taps = res_taps; p.b_resident = 1;
-        p.w = (const __nv_bfloat16*)w;
-        size_t b_all = 0;
-        p.b_res_bytes = 0;
-        for (int si = 0; si < p.nseg; ++si) {
-            Seg& s = p.seg[si];
-            const uint32_t row_bytes = (uint32_t)s.bk * 2u;
-            s.a_tx = (uint32_t)a_rows * row_bytes;
-            s.b_block_bytes = 128u * row_bytes;                 // SS fallback blocks hold M = 128 rows (rows >= Cout are TMA zero fill)
-            s.b_block_stride = (uint32_t)up1k(s.b_block_bytes);
-            s.b_base = (uint32_t)b_all;
-            b_all += (size_t)(taps - res_taps) * s.kchunks * s.b_block_stride;
-            p.b_res_bytes += (uint32_t)((taps - res_taps) * s.kchunks) * s.b_block_bytes;
-            s.kh_step16 = 0u;
-            // B operand (pixels): 8-row groups are (TW+2) rows apart in the halo box, contiguous otherwise.  The SS fallback's
-            // A operand (weights, contiguous rows) shares this descriptor high word only when the pitch is 8 rows,
-            // so halo layers keep a second high word for it.
-            const uint32_t sbo = (p.halo ? (uint32_t)(p.TW + 2) : 8u) * row_bytes, swz = s.bk == 64 ? 2u : s.bk == 32 ? 4u : 6u;
-            s.desc_hi = ((sbo >> 4) & 0x3FFFu) | (1u << 14) | (swz << 29);
-            s.desc_hi_w = (((8u * row_bytes) >> 4) & 0x3FFFu) | (1u << 14) | (swz << 29);
-            s.up = srcs[src_of[si]].up;
-            s.h_lo = H / 2;
-        }
-        p.b_stage_stride = 0;
-        p.tmem_cols = 512;
-        const size_t budget = 212 * 1024;
-        p.stg_bufs = (b_all + 2 * (size_t)128 * cout16 * 4 + 6 * (size_t)p.a_bytes <= budget) ? 2 : 1;
-        const size_t stg_bytes = (size_t)p.stg_bufs * 128 * cout16 * 4;
-        p.chunk_magic = (uint32_t)((0x100000000ull + (uint64_t)(cout16 / 16) - 1) / (uint64_t)(cout16 / 16));
-        B2_REQUIRE(b_all + stg_bytes + 4 * (size_t)p.a_bytes <= budget, "conv(ts): tile does not fit in shared memory (Cin=%d Cout=%d k=%d)", Cin, Cout, ksize);
-        size_t st_ = (budget - b_all - stg_bytes) / p.a_bytes;
-        stages = (int)(st_ > (size_t)kMaxStages ? kMaxStages : st_);
-        stages &= ~1;                                       // two rings (one per MMA warp)
-        p.num_stages = stages;
-        if (const char* dv = getenv("B2_CONV_DEBUG")) p.dbg_skip_mma = atoi(dv) == 1;
-        p.stg_off = (uint32_t)((size_t)stages * p.a_bytes + b_all);
-        L->smem = (size_t)stages * p.a_bytes + b_all + stg_bytes + 1024;
-        p.ts_steps = 0;
-        for (int si = 0; si < p.nseg; ++si) p.ts_steps += (p.halo ? 1 : taps) * p.seg[si].kchunks;
-        p.tw_log2 = 0; while ((1 << p.tw_log2) < p.TW) ++p.tw_log2;
-        p.th_log2 = 0; while ((1 << p.th_log2) < p.TH) ++p.th_log2;
-        B2_REQUIRE((1 << p.tw_log2) == p.TW && (1 << p.th_log2) == p.TH, "conv(ts): tile extents must be powers of two");
-        if (!plan_only) B2_CUDA(cudaFuncSetAttribute(conv_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 8192));   // per device: see above
-    } else {
-    // ---- resident-weight 3x3 stride-1 layers: single halo box per K chunk (halo 2, see the TS branch) when the weights and
-    //      >= 3 box stages fit; decided on the resident footprint, which does not depend on the stage layout ----
+    // ---- resident-weight 3x3 stride-1 layers: single halo box per K chunk (halo 2) when the weights and enough box stages fit;
+    //      decided on the resident footprint, which does not depend on the stage layout.  The shared-memory operand of
+    //      tcgen05.mma may start at ANY row with ANY 8-row-group pitch (the swizzle is a function of the absolute address,
+    //      DESIGN.md fact 3, profiles/r01_shift_probe.txt), so the tile's whole (TW+2) x (TH+2) box is loaded ONCE per K chunk
+    //      (180 rows instead of 3 x 144) and serves all nine taps: tap (kh, kw) starts kh * (TW+2) + kw rows in, pitch TW+2 ----
     if (p.halo == 1 && cout16 <= 256) {
         size_t w_all = 0;
         for (int si = 0; si < p.nseg; ++si) w_all += (size_t)taps * p.seg[si].kchunks * up1k((size_t)cout16 * p.seg[si].bk * 2);
@@ -1657,6 +1138,7 @@ int b2_conv_prepare_chain(void* storage, const B2ConvSrc* srcs, int nsrc, int B,
     const int want = steps_per_tile < 4 ? 4 : (steps_per_tile < kMaxStages ? steps_per_tile : kMaxStages);   // >= one tile of look-ahead
     const int s2r = (can_res && tmem2) ? fit(kTwoCta, true) : 0, s2s = tmem2 ? fit(kTwoCta, false) : 0;
     const int s1r = can_res ? fit(kOneCta, true) : 0, s1s = fit(kOneCta, false);
+    int ctas, stages;
     if (s2r >= 3) { ctas = 2; stages = s2r; p.b_resident = 1; }
     else if (s1r >= 3 || (p.halo == 2 && s1r >= 2)) { ctas = 1; stages = s1r; p.b_resident = 1; }
     else if (s2s >= 4) { ctas = 2; stages = s2s; }
@@ -1713,7 +1195,6 @@ int b2_conv_prepare_chain(void* storage, const B2ConvSrc* srcs, int nsrc, int B,
         if ((p.c2_buf_off | p.c2_buf_bytes) & 1023u) { b2_set_error("conv(chain): staged-tile buffers must be 1 KiB aligned"); return B2_ERR_UNSUPPORTED; }
         for (int i = 0; i < p.c2_nblk; ++i) p.b_res_bytes += p.c2_w_bytes[i];
         L->smem += chain_bytes;
-    }
     }
     p.out = (__nv_bfloat16*)out; p.out_cstride = out_cstride; p.out_coff = out_coff;
     p.res = (const __nv_bfloat16*)residual; p.res_cstride = res_cstride; p.res_coff = res_coff;
@@ -1787,7 +1268,7 @@ int b2_conv_prepare_chain(void* storage, const B2ConvSrc* srcs, int nsrc, int B,
         const cuuint64_t K = (cuuint64_t)ksize * ksize * Cin;
         const cuuint64_t dimsb[2] = {K, (cuuint64_t)Cout};
         const cuuint64_t stridesb[1] = {K * 2};
-        const cuuint32_t boxb[2] = {(cuuint32_t)s.bk, (cuuint32_t)(p.ts ? 128 : p.n_tile)};
+        const cuuint32_t boxb[2] = {(cuuint32_t)s.bk, (cuuint32_t)p.n_tile};
         const cuuint32_t es[2] = {1, 1};
         CUresult r = encode(&s.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w, dimsb, stridesb, boxb, es,
                             CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1843,7 +1324,7 @@ int b2_conv_set_head_epilogue(void* storage, int epi, float* out_f32) {
         return B2_OK;
     }
     B2_REQUIRE(L->p.n_tiles == 1 && (epi != 1 || L->p.Cout == 64) && out_f32, "conv: head epilogue needs one N tile (DFL: exactly 64 channels)");
-    B2_REQUIRE(!L->p.ts && L->p.halo == 0, "conv: head epilogues are implemented for 1x1 convs in conv_tc_kernel only");
+    B2_REQUIRE(L->p.halo == 0, "conv: head epilogues are implemented for 1x1 convs in conv_tc_kernel only");
     L->p.mma_warps = 1;
     L->p.epi = epi; L->p.out_f32 = out_f32;
     return B2_OK;
@@ -1853,7 +1334,6 @@ void b2_count_launch(int n);
 
 int b2_conv_launch(const void* storage, cudaStream_t stream) {
     const B2ConvLaunch* L = reinterpret_cast<const B2ConvLaunch*>(storage);
-    if (L->p.ts) { conv_ts_kernel<<<L->grid, kTsThreads, L->smem, stream>>>(L->p); B2_CUDA(cudaGetLastError()); b2_count_launch(1); return B2_OK; }
     // programmatic dependent launch: this grid's prologue overlaps the tail of the previous kernel of the stream when that
     // kernel is a conv_tc_kernel too (it calls griddepcontrol.launch_dependents); otherwise the attribute changes nothing
     static const bool pdl = [] { const char* v = getenv("B2_CONV_PDL"); return !(v && atoi(v) == 0); }();
