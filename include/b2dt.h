@@ -272,6 +272,34 @@ int b2_iou_cost(const float* boxes_a, const float* boxes_b, const float* scores_
  * Exact optimum (float64 shortest augmenting paths), one CTA per problem. */
 int b2_linear_assignment(const float* cost, const int32_t* na, const int32_t* nb, int S, int n_max, int m_max, float thresh,
                          int32_t* x_out, int32_t* y_out, void* stream);
+/* The same solver on a float64 cost [S][n_max][m_max] with a float64 threshold (lap.lapjv works in double: the BoT-SORT ReID cost
+ * is float64 and can hold entries closer to the threshold than float32 resolves). */
+int b2_linear_assignment_f64(const double* cost, const int32_t* na, const int32_t* nb, int S, int n_max, int m_max, double thresh,
+                             int32_t* x_out, int32_t* y_out, void* stream);
+/* BOTSORT.get_dists with ReID (ultralytics/trackers/bot_sort.py:154-232, matching.embedding_distance):
+ *   d    = iou_distance (float32, as b2_iou_cost);  mask = d > prox_limit (float32; prox_limit = float32(1 - proximity_thresh))
+ *   d    = fuse_score(d) when scores_b is given (float32)
+ *   emb  = max(0, cdist(feat_a, feat_b, 'cosine')) / 2 in float64;  emb[emb > app_limit] = 1 (app_limit = 1 - appearance_thresh);
+ *   emb[mask] = 1;  cost = minimum(d, emb) float64 [S][n_max][m_max] (entries outside a problem's corner are not touched).
+ * feat_a: track smooth features [S][n_max][D], feat_b: detection features [S][m_max][D], fp32. */
+int b2_botsort_cost(const float* boxes_a, const float* boxes_b, const float* scores_b, const int32_t* na, const int32_t* nb,
+                    const float* feat_a, const float* feat_b, int D, int S, int n_max, int m_max, float prox_limit, double app_limit,
+                    double* cost, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * BoT-SORT ReID on the detector's own features (botsort.yaml with_reid: True, model: auto)
+ * ---------------------------------------------------------------------------------------------- */
+/* get_obj_feats (models/yolo/detect/predict.py): out[b][k][0..s) = row of kept detection k of image b in the Detect input map of its
+ * level, averaged over groups of C_l / s consecutive channels (fp32, not normalised).  Level l (host arrays, Detect order): NHWC
+ * bf16 buffer level_ptr[l] [B][h][w][cstride], channels [coff, coff + C); anchor ids count the levels' h*w pixels in that order.
+ * det_idx [B][max_det] (b2_nms out_idx), det_count [B].  Every C_l must be a multiple of s.  Rows k >= det_count[b] are not written. */
+int b2_reid_gather(const void* const* level_ptr, const int* level_h, const int* level_w, const int* level_cstride, const int* level_coff,
+                   const int* level_c, int n_levels, const int32_t* det_idx, const int32_t* det_count, int B, int max_det, int s,
+                   float* out, void* stream);
+/* BOTrack.update_features (bot_sort.py) for N rows, float32: curr [N][D] /= |curr| in place; where has_smooth[r] (NULL: no row)
+ * smooth = 0.9 smooth + 0.1 curr, otherwise smooth = curr; then smooth /= |smooth| (a first smooth is the same vector as curr in
+ * the reference, so curr receives that renormalisation too). */
+int b2_reid_update(float* curr, float* smooth, const uint8_t* has_smooth, int N, int D, void* stream);
 
 #ifdef __cplusplus
 }

@@ -73,6 +73,10 @@ SIGNATURES = {
     "b2_kf_gating": (c_int, [c_int, _P, _P, c_int, _P, c_int, c_int, c_int, _P, _P]),
     "b2_iou_cost": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P, _P]),
     "b2_linear_assignment": (c_int, [_P, _P, _P, c_int, c_int, c_int, c_float, _P, _P, _P]),
+    "b2_linear_assignment_f64": (c_int, [_P, _P, _P, c_int, c_int, c_int, C.c_double, _P, _P, _P]),
+    "b2_botsort_cost": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, C.c_double, _P, _P]),
+    "b2_reid_gather": (c_int, [_P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_int, _P, _P]),
+    "b2_reid_update": (c_int, [_P, _P, _P, c_int, c_int, _P]),
 }
 
 B2_OK, B2_ERR_ARG, B2_ERR_CUDA, B2_ERR_STATE, B2_ERR_UNSUPPORTED = 0, -1, -2, -3, -4

@@ -1,4 +1,4 @@
-"""Upstream tracker plug-in (ByteTrack, BoT-SORT without ReID) over the B200 kernels: mirror of ``ultralytics/trackers/byte_tracker.py`` (STrack
+"""Upstream tracker plug-in (ByteTrack, BoT-SORT with or without ReID) over the B200 kernels: mirror of ``ultralytics/trackers/byte_tracker.py`` (STrack
 :14-237, BYTETracker :240-485), ``trackers/utils/matching.py`` (linear_assignment :20-63, iou_distance :66-113, fuse_score
 :135-157) and the ``trackers/track.py`` callback contract (:72-102: ``tracker.update(boxes) -> (k, 8)`` rows
 ``[x1, y1, x2, y2, track_id, score, cls, idx]``, ``Results.update(boxes=rows[:, :-1])``).
@@ -9,9 +9,16 @@ Same names, arguments and control flow as the reference; the numeric work of a f
 dependency), ``b2_kf_update`` / ``b2_kf_initiate`` batched over the matches of a stage (the reference updates matched tracks one
 by one; the stages only ever look at tracks that were NOT matched before, so batching per stage is the same computation).
 Track state is float32 on the device (float64 numpy in the reference).  No CPU fallback: every call needs the CUDA library.
+
+BoT-SORT ReID (botsort.yaml ``with_reid: True`` with ``model: auto``, bot_sort.py BOTrack.update_features, BOTSORT.get_dists,
+matching.embedding_distance): the appearance vectors are the detector's own Detect-input features (``Results.feats``, gathered
+by ``b2_reid_gather``) and stay on the device as float32 rows; ``b2_reid_update`` normalises / smooths them for all of a stage's
+pairs in one launch, ``b2_botsort_cost`` forms the combined float64 cost of stages 1 and 3 and ``b2_linear_assignment_f64``
+solves it.  A separate ReID network (``model: yolo11n-cls.pt``, ...) is not provided.
 """
 from __future__ import annotations
 
+from collections import deque
 from types import SimpleNamespace
 
 import numpy as np
@@ -67,15 +74,16 @@ def linear_assignment(cost_matrix, thresh, use_lap=True):
     cost_matrix = np.asarray(cost_matrix)
     if cost_matrix.size == 0:
         return np.empty((0, 2), dtype=int), tuple(range(cost_matrix.shape[0])), tuple(range(cost_matrix.shape[1]))
-    x, y = linear_assignment_device(torch.as_tensor(np.ascontiguousarray(cost_matrix, np.float32), device="cuda")[None], thresh)
+    dt = np.float64 if cost_matrix.dtype == np.float64 else np.float32          # lapjv solves a float64 cost as it is
+    x, y = linear_assignment_device(torch.as_tensor(np.ascontiguousarray(cost_matrix, dt), device="cuda")[None], thresh)
     x, y = x[0].cpu().numpy(), y[0].cpu().numpy()
     matches = [[ix, int(mx)] for ix, mx in enumerate(x) if mx >= 0]
     return matches, np.where(x < 0)[0], np.where(y < 0)[0]
 
 
 def linear_assignment_device(cost, thresh, na=None, nb=None):
-    """Batched form: cost CUDA float32 [S][n_max][m_max] (problem s uses its na[s] x nb[s] corner) -> (x [S][n_max], y [S][m_max])
-    int32 CUDA tensors, -1 = unmatched."""
+    """Batched form: cost CUDA float32 or float64 [S][n_max][m_max] (problem s uses its na[s] x nb[s] corner) -> (x [S][n_max],
+    y [S][m_max]) int32 CUDA tensors, -1 = unmatched."""
     import torch
 
     _lib.require_cuda()
@@ -83,9 +91,52 @@ def linear_assignment_device(cost, thresh, na=None, nb=None):
     S, n, m = cost.shape
     x = torch.empty((S, n), dtype=torch.int32, device="cuda")
     y = torch.empty((S, m), dtype=torch.int32, device="cuda")
-    _lib.check(lib.b2_linear_assignment(_lib.ptr(cost.contiguous()), _lib.ptr(na), _lib.ptr(nb), S, n, m, float(thresh), _lib.ptr(x), _lib.ptr(y),
-                                        _lib.stream_ptr()))
+    solve = lib.b2_linear_assignment_f64 if cost.dtype == torch.float64 else lib.b2_linear_assignment
+    if cost.dtype not in (torch.float32, torch.float64):
+        raise TypeError(f"linear_assignment: cost dtype {cost.dtype} (float32 or float64)")
+    _lib.check(solve(_lib.ptr(cost.contiguous()), _lib.ptr(na), _lib.ptr(nb), S, n, m, float(thresh), _lib.ptr(x), _lib.ptr(y), _lib.stream_ptr()))
     return x, y
+
+
+def botsort_distance(tracks, detections, scores, proximity_thresh, appearance_thresh):
+    """BOTSORT.get_dists with ReID (bot_sort.py:154-232, matching.embedding_distance) in one b2_botsort_cost launch: the IoU
+    distance (fused with ``scores`` when given) where it is below the combined appearance / proximity gate of the float64 cosine
+    distance between track ``smooth_feat`` and detection ``curr_feat``.  Returns the float64 (N, M) matrix."""
+    import torch
+
+    n, m = len(tracks), len(detections)
+    if n == 0 or m == 0:
+        return np.zeros((n, m), dtype=np.float64)
+    _lib.require_cuda()
+    lib = _lib.load()
+    a = torch.as_tensor(_boxes_of(tracks), device="cuda")
+    b = torch.as_tensor(_boxes_of(detections), device="cuda")
+    sc = None if scores is None else torch.as_tensor(np.ascontiguousarray(scores, np.float32), device="cuda")
+    fa = torch.stack([t.smooth_feat for t in tracks])
+    fb = torch.stack([d.curr_feat for d in detections])
+    if fa.shape[1] != fb.shape[1]:
+        raise ValueError(f"feature widths differ: tracks {fa.shape[1]}, detections {fb.shape[1]}")
+    cost = torch.empty((n, m), dtype=torch.float64, device="cuda")
+    # dists > (1 - proximity_thresh) compares a float32 matrix with a Python float: NumPy 2 rounds the scalar to float32;
+    # emb > (1 - appearance_thresh) compares float64 with float64
+    _lib.check(lib.b2_botsort_cost(_lib.ptr(a), _lib.ptr(b), _lib.ptr(sc), None, None, _lib.ptr(fa), _lib.ptr(fb), fa.shape[1], 1, n, m,
+                                   float(np.float32(1 - proximity_thresh)), float(1 - appearance_thresh), _lib.ptr(cost), _lib.stream_ptr()))
+    return cost.cpu().numpy()
+
+
+def reid_update(curr, smooth=None, has_smooth=None):
+    """BOTrack.update_features for every row of ``curr`` (CUDA float32 [N][D], normalised in place) in one b2_reid_update launch.
+    ``smooth``: the rows' previous smooth features (float32 [N][D], updated in place) with ``has_smooth`` (bool per row) telling
+    which exist; None: first features only.  Returns (curr, smooth)."""
+    import torch
+
+    _lib.require_cuda()
+    N, D = curr.shape
+    if smooth is None:
+        smooth = torch.empty_like(curr)
+    mask = None if has_smooth is None else torch.as_tensor(np.asarray(has_smooth, np.uint8), device="cuda")
+    _lib.check(_lib.load().b2_reid_update(_lib.ptr(curr), _lib.ptr(smooth), _lib.ptr(mask), N, D, _lib.stream_ptr()))
+    return curr, smooth
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -230,6 +281,8 @@ DEFAULT_ARGS = dict(tracker_type="bytetrack", track_high_thresh=0.25, track_low_
 class BYTETracker:
     """byte_tracker.py:240-485.  ``args``: a namespace / dict with the bytetrack.yaml keys (None: the yaml's defaults)."""
 
+    reid = False                # BOTSORT with_reid: detections carry appearance features
+
     def __init__(self, args=None, frame_rate=30):
         if args is None:
             args = DEFAULT_ARGS
@@ -254,7 +307,7 @@ class BYTETracker:
         return [STrack(xywh, s, c) for (xywh, s, c) in zip(bboxes, np.asarray(results.conf), np.asarray(results.cls))]
 
     def get_dists(self, tracks, detections):
-        """iou_distance (+ fuse_score) in one launch."""
+        """Cost of stages 1 and 3: iou_distance (+ fuse_score) in one launch."""
         return iou_distance(tracks, detections, [d.score for d in detections] if self.args.fuse_score else None)
 
     def multi_predict(self, tracks):
@@ -277,6 +330,8 @@ class BYTETracker:
         ``touched`` collects the tracks, re-found ones flagged."""
         if not pairs:
             return
+        if self.reid:
+            self._update_features(pairs)
         means, covs = self.kalman_filter.update(np.asarray([t.mean for t, _ in pairs]), np.asarray([t.covariance for t, _ in pairs]),
                                                 np.asarray([t.convert_coords(d.tlwh) for t, d in pairs], dtype=np.float32))
         for (trk, det), m, c in zip(pairs, means, covs):
@@ -287,14 +342,16 @@ class BYTETracker:
                 trk.re_activate(det, self.frame_id, m, c, new_id=False)
             touched.append((trk, not was_tracked))
 
-    def _stage(self, tracks, dets, thresh, fuse):
-        """One association stage: cost launch + assignment launch -> (pairs, unmatched track indices, unmatched detection indices)."""
-        cost = iou_distance(tracks, dets, [d.score for d in dets] if fuse else None)
+    def _stage(self, tracks, dets, thresh, dists):
+        """One association stage: cost launch (``dists(tracks, dets)``) + assignment launch -> (pairs, unmatched track indices,
+        unmatched detection indices)."""
+        cost = dists(tracks, dets)
         matches, free_t, free_d = linear_assignment(cost, thresh=thresh)
         return [(tracks[a], dets[b]) for a, b in matches], list(free_t), list(free_d)
 
     def update(self, results, img=None, feats=None):
-        """:299-410.  results: a ``Boxes``-like object on the host (``.conf``, ``.cls``, ``.xywh``, boolean-mask indexing).
+        """:299-410.  results: a ``Boxes``-like object on the host (``.conf``, ``.cls``, ``.xywh``, boolean-mask indexing);
+        feats: the rows' appearance vectors (``Results.feats``; read by BOTSORT with ReID only), split like the boxes.
         Stages as in the reference: high-score boxes against tracked + lost tracks (threshold ``match_thresh``, scores fused when
         ``fuse_score``), low-score boxes against the still-unmatched TRACKED tracks (plain IoU, 0.5), the remaining high-score
         boxes against the one-frame-old unconfirmed tracks (0.7), then births, time-outs and de-duplication."""
@@ -303,7 +360,10 @@ class BYTETracker:
         conf = np.asarray(results.conf)
         high = conf >= cfg_.track_high_thresh
         low = (conf > cfg_.track_low_thresh) & (conf < cfg_.track_high_thresh)
-        dets_high, dets_low = self.init_track(results[high]), None
+        feats_high = feats_low = None
+        if self.reid:
+            feats_high, feats_low = self._split_feats(feats, len(conf), high, low)
+        dets_high = self.init_track(results[high], feats_high)
         confirmed = [t for t in self.tracked_stracks if t.is_activated]
         tentative = [t for t in self.tracked_stracks if not t.is_activated]
         pool = self.joint_stracks(confirmed, self.lost_stracks)
@@ -317,12 +377,12 @@ class BYTETracker:
             STrack.multi_gmc(tentative, warp)
         touched, newly_lost, dropped = [], [], []
         # stage 1
-        pairs, free_t, free_d = self._stage(pool, dets_high, cfg_.match_thresh, cfg_.fuse_score)
+        pairs, free_t, free_d = self._stage(pool, dets_high, cfg_.match_thresh, self.get_dists)
         self._apply(pairs, touched)
         # stage 2: only tracks that were being tracked compete for the low-score boxes; the rest of stage 1's leftovers stay lost
-        dets_low = self.init_track(results[low])
+        dets_low = self.init_track(results[low], feats_low)
         still_tracked = [pool[k] for k in free_t if pool[k].state == TrackState.Tracked]
-        pairs, free_t2, _ = self._stage(still_tracked, dets_low, 0.5, False)
+        pairs, free_t2, _ = self._stage(still_tracked, dets_low, 0.5, iou_distance)
         self._apply(pairs, touched)
         for k in free_t2:
             trk = still_tracked[k]
@@ -331,7 +391,7 @@ class BYTETracker:
                 newly_lost.append(trk)
         # stage 3
         leftovers = [dets_high[k] for k in free_d]
-        pairs, free_u, free_d = self._stage(tentative, leftovers, 0.7, cfg_.fuse_score)
+        pairs, free_u, free_d = self._stage(tentative, leftovers, 0.7, self.get_dists)
         self._apply(pairs, touched)
         for k in free_u:
             tentative[k].mark_removed()
@@ -435,9 +495,16 @@ class GMC:
 
 
 class BOTrack(STrack):
-    """bot_sort.py:20-151 without appearance features: XYWH filter, both size velocities zeroed while a track is not Tracked."""
+    """bot_sort.py:20-151: XYWH filter, both size velocities zeroed while a track is not Tracked.  With ReID: ``curr_feat`` /
+    ``smooth_feat`` (CUDA float32 rows) and the last 50 ``features``, set by BOTSORT in batches (``b2_reid_update``)."""
 
     shared_kalman = None
+
+    def __init__(self, xywh, score, cls):
+        super().__init__(xywh, score, cls)
+        self.smooth_feat = self.curr_feat = None
+        self.features = deque([], maxlen=50)
+        self.alpha = 0.9
 
     @staticmethod
     def multi_predict(stracks):
@@ -476,8 +543,9 @@ BOTSORT_DEFAULT_ARGS = dict(DEFAULT_ARGS, tracker_type="botsort", gmc_method="sp
 
 
 class BOTSORT(BYTETracker):
-    """bot_sort.py:154-232 with ``with_reid=False`` (the yaml's default): ByteTrack's association on the XYWH filter plus global
-    motion compensation from the frame handed to ``update(results, img)``."""
+    """bot_sort.py:154-232: ByteTrack's association on the XYWH filter plus global motion compensation from the frame handed to
+    ``update(results, img, feats)``.  ``with_reid=True`` with ``model: auto``: ``feats`` (n, D) are the detections' appearance
+    vectors and stages 1 and 3 use the combined IoU / appearance cost (``botsort_distance``)."""
 
     def __init__(self, args=None, frame_rate=30):
         from .kalman_filter import KalmanFilterXYWH
@@ -487,8 +555,9 @@ class BOTSORT(BYTETracker):
             args = BOTSORT_DEFAULT_ARGS
         if isinstance(args, dict):
             args = SimpleNamespace(**{**BOTSORT_DEFAULT_ARGS, **args})
-        if getattr(args, "with_reid", False):
-            raise NotImplementedError("BoT-SORT ReID (appearance embeddings) is outside the hot path")
+        self.reid = bool(getattr(args, "with_reid", False))
+        if self.reid and getattr(args, "model", "auto") != "auto":
+            raise NotImplementedError(f"BoT-SORT ReID model {args.model!r}: only the detector's own features (model: auto) are provided")
         super().__init__(args, frame_rate)
         self.gmc = GMC(method=args.gmc_method)
         self.proximity_thresh, self.appearance_thresh = args.proximity_thresh, args.appearance_thresh
@@ -500,11 +569,49 @@ class BOTSORT(BYTETracker):
         return kf
 
     def init_track(self, results, img=None):
+        """``img``: with ReID, the rows' features (CUDA float32, a private copy): normalised as the BOTrack constructor's
+        update_features does, in one launch."""
         if len(results) == 0:
             return []
         bboxes = np.asarray(results.xywh, dtype=np.float32)
         bboxes = np.concatenate([bboxes, np.arange(len(bboxes), dtype=np.float32).reshape(-1, 1)], axis=-1)
-        return [BOTrack(xywh, s, c) for (xywh, s, c) in zip(bboxes, np.asarray(results.conf), np.asarray(results.cls))]
+        tracks = [BOTrack(xywh, s, c) for (xywh, s, c) in zip(bboxes, np.asarray(results.conf), np.asarray(results.cls))]
+        if self.reid and img is not None:
+            curr, smooth = reid_update(img)
+            for t, c, sm in zip(tracks, curr, smooth):
+                t.curr_feat, t.smooth_feat = c, sm
+                t.features.append(c)
+        return tracks
+
+    def get_dists(self, tracks, detections):
+        if not self.reid:
+            return super().get_dists(tracks, detections)
+        return botsort_distance(tracks, detections, [d.score for d in detections] if self.args.fuse_score else None,
+                                self.proximity_thresh, self.appearance_thresh)
+
+    @staticmethod
+    def _split_feats(feats, n, high, low):
+        """feats[remain_inds], feats[inds_second] (byte_tracker.py update) as CUDA float32 copies."""
+        import torch
+
+        if feats is None:
+            raise ValueError("BOTSORT(with_reid=True).update needs the detections' features (Results.feats)")
+        f = torch.as_tensor(feats, dtype=torch.float32, device="cuda")
+        if f.ndim != 2 or f.shape[0] != n:
+            raise ValueError(f"feats of shape {tuple(f.shape)} for {n} detections")
+        pick = lambda m: f.index_select(0, torch.as_tensor(np.flatnonzero(m), device="cuda"))
+        return pick(high), pick(low)
+
+    def _update_features(self, pairs):
+        """update_features(det.curr_feat) of every track of one stage's pairs (BOTrack.update / re_activate) in one launch."""
+        import torch
+
+        curr = torch.stack([d.curr_feat for _, d in pairs])
+        smooth = torch.stack([t.smooth_feat if t.smooth_feat is not None else d.curr_feat for t, d in pairs])
+        curr, smooth = reid_update(curr, smooth, [t.smooth_feat is not None for t, _ in pairs])
+        for (t, _), c, sm in zip(pairs, curr, smooth):
+            t.curr_feat, t.smooth_feat = c, sm
+            t.features.append(c)
 
     def multi_predict(self, tracks):
         BOTrack.multi_predict(tracks)
@@ -523,7 +630,7 @@ def update_results(trackers, results, is_stream=True):
     for i, result in enumerate(results):
         tracker = trackers[i if is_stream else 0]
         det = result.boxes.cpu().numpy()
-        tracks = tracker.update(det, getattr(result, "orig_img", None))
+        tracks = tracker.update(det, getattr(result, "orig_img", None), getattr(result, "feats", None))
         if len(tracks) == 0:
             continue
         result.update(boxes=tracks[:, :-1])

@@ -493,6 +493,24 @@ class Engine:
         buf, off, c = self.plan.named[name] if isinstance(name, str) else self.plan.loc[name]
         return self.buffer(buf)[..., off:off + c].float().permute(0, 3, 1, 2).contiguous()
 
+    def detect_inputs(self):
+        """The feature maps that feed Detect (its ``f`` layers, in ``f`` order) as they stand after the last forward: one
+        (device pointer, h, w, buffer channel stride, channel offset, C) per level.  C is Detect's own input width (``ch``), so
+        the zero channels a padded plan adds after it are not part of the slice.  These are the maps the reference's ReID
+        hook reads (trackers/track.py on_predict_start, ``model: auto``); they stay valid until the next forward."""
+        det = self.spec["layers"][-1]
+        s = min(det["ch"])
+        if any(c % s for c in det["ch"]):
+            raise NotImplementedError(f"Detect input widths {det['ch']}: get_obj_feats needs every width to be a multiple of {s}")
+        out = []
+        for f, c in zip(det["f"], det["ch"]):
+            buf, coff, _ = self.plan.loc[f]
+            h, w, cstride = self.plan.bufs[buf]
+            p, hh, ww, cc = C.c_void_p(), C.c_int(), C.c_int(), C.c_int()
+            _lib.check(self.lib.b2_engine_buffer(self._h, buf, C.byref(p), C.byref(hh), C.byref(ww), C.byref(cc)))
+            out.append((p.value, h, w, cstride, coff, c))
+        return out
+
     def level_logits(self, l):
         """[B][h*w][lstride] bf16 view of Detect level ``l`` (64 DFL bins, then nc class logits)."""
         return _view_bf16(self.level_ptrs[l], (self.B, self.level_h[l] * self.level_w[l], self.lstride))

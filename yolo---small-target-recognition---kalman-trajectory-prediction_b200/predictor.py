@@ -11,6 +11,7 @@ with the three stages executed by the CUDA library: stem-fused preprocess + forw
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 import os
 import time
@@ -283,6 +284,7 @@ class DetectPipeline:
         e = self.engine
         self.post = ops.DetectPost(batch, e.level_h, e.level_w, e.level_stride, e.nc, e.lstride, max_det=max_det)
         self.B, self.H, self.W = batch, H, W
+        self.feats = None
 
     def __call__(self, frames_u8, conf, iou, pad_top=0, pad_left=0, orig_hw=None, classes_mask=None, agnostic=False,
                  mode="exact", stream=None):
@@ -308,6 +310,23 @@ class DetectPipeline:
     def nms(self, iou, orig_hw=None, agnostic=False, mode="exact", stream=None):
         scale = scale_params((self.H, self.W), orig_hw) if orig_hw is not None else None
         return self.post.nms(iou, agnostic=agnostic, mode=mode, scale=scale, stream=stream)
+
+    def embed(self, stream=None):
+        """get_obj_feats (models/yolo/detect/predict.py) for the detections ``nms`` kept: [B][max_det][s] fp32 device tensor, row k
+        of image b valid for k < count[b].  Reads the Detect inputs in the engine arena, so it must follow ``nms`` on the same
+        stream before the next forward."""
+        import torch
+
+        lv = self.engine.detect_inputs()
+        s = min(c for *_, c in lv)
+        if self.feats is None:
+            self.feats = torch.empty((self.B, self.post.max_det, s), dtype=torch.float32, device="cuda")
+        n = len(lv)
+        arr = lambda k: (C.c_int * n)(*[d[k] for d in lv])
+        _lib.check(self.engine.lib.b2_reid_gather((C.c_void_p * n)(*[d[0] for d in lv]), arr(1), arr(2), arr(3), arr(4), arr(5), n,
+                                                  _lib.ptr(self.post.out_idx), _lib.ptr(self.post.out_count), self.B, self.post.max_det, s,
+                                                  _lib.ptr(self.feats), _lib.stream_ptr(stream)))
+        return self.feats
 
 
 class YOLO:
@@ -375,6 +394,7 @@ class YOLO:
             return gen() if stream else list(gen())
 
         a = {**self.overrides, **kwargs}
+        want_feats = bool(a.pop("_feats", False))      # internal (YOLO.track with BoT-SORT ReID): Results.feats per image
         if a.get("predictor") is not None:
             # engine/model.py:549 swaps the predictor class; this facade IS the predictor -- to put the engine behind an installed
             # Ultralytics model use b200dt.ultra_plugin.predictor_class()
@@ -403,12 +423,15 @@ class YOLO:
             B, _, H, W = x.shape
             pipe = self._pipe(B, H, W, max_det)
             dets, counts = pipe.run_tensor(x, conf, iou, (H, W), cmask, a["agnostic_nms"], a["nms_mode"])
+            feats = pipe.embed() if want_feats else None
             cnt = counts.cpu().tolist()
             ms = (time.perf_counter() - t0) * 1e3 / B
             imgs = (x.float().permute(0, 2, 3, 1).flip(-1) * 255).to(torch.uint8).cpu().numpy()    # loaders convert_torch2numpy_batch
             for b in range(B):
                 results.append(Results(imgs[b], f"image{b}.jpg", self.names, dets[b, :cnt[b]].clone(),
                                        {"preprocess": 0.0, "inference": ms, "postprocess": 0.0}))
+                if want_feats:
+                    results[-1].feats = feats[b, :cnt[b]].clone()
         else:
             frames = [source] if isinstance(source, np.ndarray) else list(source)
             if not frames:
@@ -430,11 +453,14 @@ class YOLO:
                     raise ValueError(f"letterboxed size {H}x{W} is not a multiple of 32")
                 pipe = self._pipe(len(idxs), H, W, max_det)
                 dets, counts = pipe(batch, conf, iou, top, left, (h0, w0), cmask, a["agnostic_nms"], a["nms_mode"])
+                feats = pipe.embed() if want_feats else None          # before the next group's forward reuses the arena
                 cnt = counts.cpu().tolist()
                 ms = (time.perf_counter() - t0) * 1e3 / len(idxs)
                 for j, i in enumerate(idxs):
                     out[i] = Results(frames[i], f"image{i}.jpg", self.names, dets[j, :cnt[j]].clone(),
                                      {"preprocess": 0.0, "inference": ms, "postprocess": 0.0})
+                    if want_feats:
+                        out[i].feats = feats[j, :cnt[j]].clone()
             results = out
         if a.get("verbose"):
             for r in results:
@@ -443,13 +469,23 @@ class YOLO:
 
     def track(self, source=None, stream=False, persist=False, **kwargs):
         """engine/model.py:559-591 + trackers/track.py: predict with conf 0.1 by default (ByteTrack wants the low-confidence boxes),
-        then the tracker's update attaches ids (``Results.boxes.id``).  ``tracker``: 'bytetrack.yaml' or a dict of its keys.
+        then the tracker's update attaches ids (``Results.boxes.id``).  ``tracker``: 'bytetrack.yaml' / 'botsort.yaml' (the defaults),
+        the path of a tracker YAML file (its keys over the defaults of its ``tracker_type``) or a dict of the keys.  BoT-SORT with
+        ``with_reid: True`` (``model: auto``) gets each detection's appearance vector from the detector (``Results.feats``).
         A list of frames is one video, walked in order by ONE tracker (the reference's non-stream datasets); ``persist=True`` keeps
         the tracker between calls."""
         from . import byte_tracker
 
         tracker = kwargs.pop("tracker", "bytetrack.yaml")
         cls = byte_tracker.BYTETracker
+        if isinstance(tracker, (str, os.PathLike)) and str(tracker) not in ("bytetrack.yaml", "botsort.yaml") and os.path.isfile(tracker):
+            import yaml
+
+            with open(tracker, encoding="utf-8") as fh:
+                tracker = yaml.safe_load(fh) or {}
+            kind = tracker.get("tracker_type")
+            if kind not in ("bytetrack", "botsort"):
+                raise AssertionError(f"Only 'bytetrack' and 'botsort' are supported for now, but got '{kind}'")
         if isinstance(tracker, str):
             if "botsort" in tracker:
                 cls = byte_tracker.BOTSORT
@@ -461,6 +497,8 @@ class YOLO:
         kwargs["conf"] = kwargs.get("conf") or 0.1
         if not (persist and getattr(self, "trackers", None)):
             self.trackers = [cls(tracker, frame_rate=30)]
+        if self.trackers[0].reid:
+            kwargs["_feats"] = True
         if isinstance(source, (str, os.PathLike)) or (isinstance(source, (list, tuple)) and source and isinstance(source[0], (str, os.PathLike))):
             # file sources: frames arrive batch by batch; the tracker is reset when the file changes (track.py:87-89, persist=False)
             def gen():
