@@ -96,6 +96,12 @@ int b2_preprocess_u8(const uint8_t* frames, int B, int src_h, int src_w, int H, 
                      float* out_bchw, void* stream);
 /* cv2.resize(INTER_LINEAR) on uint8 HWC (data/augment.py:1718): fixed-point bilinear identical to OpenCV. */
 int b2_resize_bilinear_u8(const uint8_t* src, int B, int sh, int sw, uint8_t* dst, int dh, int dw, void* stream);
+/* LetterBox (data/augment.py:1692-1733) for a ragged batch: image b is src_h x src_w HWC BGR at byte offset src_off[b] of `src`
+ * (16-byte aligned offsets take the vector copy path); it is resized to rh x rw with the arithmetic of b2_resize_bilinear_u8
+ * (copied when the shape is unchanged) and placed at (top, left) of canvas b; everything else is 114.
+ * src_off: device int64 [B]; geom: device int32 [B][6] {src_h, src_w, rh, rw, top, left}; canvas: [B][H][W][3] uint8,
+ * W a multiple of 16, at most 4096.  A placement that does not fit the canvas leaves that canvas at 114. */
+int b2_letterbox_u8(const uint8_t* src, const int64_t* src_off, const int32_t* geom, int B, int H, int W, uint8_t* canvas, void* stream);
 
 /* SPPF pooling (block.py:237-241): y1 = maxpool5(x), y2 = maxpool5(y1), y3 = maxpool5(y2) (stride 1, pad 2).
  * buf: [B][H][W][cstride] bf16; reads channels [coff, coff+C), writes [coff+C, coff+4C). */
@@ -144,6 +150,11 @@ int b2_nms(const float* cand, const int32_t* cand_idx, const int32_t* cand_count
            float iou_thres, int max_det, int max_nms, int agnostic, float max_wh, int mode,
            float gain, float pad_x, float pad_y, float orig_w, float orig_h, int do_scale,
            float* out, int32_t* out_count, int32_t* out_idx, void* workspace, size_t workspace_bytes, void* stream);
+/* b2_nms with scale_boxes + clip_boxes per image: scale is a device float [B][5] {gain, pad_x, pad_y, orig_w, orig_h}, row b
+ * applied to image b with the same operations as the scalar epilogue (a batch of frames of different original shapes). */
+int b2_nms_scaled(const float* cand, const int32_t* cand_idx, const int32_t* cand_count, int cand_cap, int B,
+                  float iou_thres, int max_det, int max_nms, int agnostic, float max_wh, int mode, const float* scale,
+                  float* out, int32_t* out_count, int32_t* out_idx, void* workspace, size_t workspace_bytes, void* stream);
 size_t b2_nms_workspace_bytes(int B, int cand_cap);
 
 /* ------------------------------------------------------------------------------------------------

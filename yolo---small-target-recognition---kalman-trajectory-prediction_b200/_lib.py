@@ -31,6 +31,7 @@ SIGNATURES = {
     "b2_stem_f32": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, c_int, c_int, _P]),
     "b2_preprocess_u8": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "b2_resize_bilinear_u8": (c_int, [_P, c_int, c_int, c_int, _P, c_int, c_int, _P]),
+    "b2_letterbox_u8": (c_int, [_P, _P, _P, c_int, c_int, c_int, _P, _P]),
     "b2_sppf_pool": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P]),
     "b2_upsample_slice": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, _P]),
     "b2_decode": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, _P, _P, _P, _P, c_int, _P, _P]),
@@ -38,6 +39,8 @@ SIGNATURES = {
     "b2_candidates_from_dense": (c_int, [_P, c_int, c_int, c_int, c_int, c_float, _P, _P, _P, _P, c_int, _P]),
     "b2_nms": (c_int, [_P, _P, _P, c_int, c_int, c_float, c_int, c_int, c_int, c_float, c_int,
                        c_float, c_float, c_float, c_float, c_float, c_int, _P, _P, _P, _P, c_size_t, _P]),
+    "b2_nms_scaled": (c_int, [_P, _P, _P, c_int, c_int, c_float, c_int, c_int, c_int, c_float, c_int, _P,
+                              _P, _P, _P, _P, c_size_t, _P]),
     "b2_nms_workspace_bytes": (c_size_t, [c_int, c_int]),
     "b2_engine_create": (c_int, [_P, c_int, _P, c_size_t, c_int, c_int, c_int, C.POINTER(_P)]),
     "b2_engine_destroy": (c_int, [_P]),

@@ -293,6 +293,7 @@ struct NmsParams {
     const float* cand; const int32_t* cand_idx; const int32_t* cand_count; int cand_cap, B;
     float iou_thres; int max_det, max_nms, agnostic; float max_wh; int mode;
     float gain, pad_x, pad_y, orig_w, orig_h; int do_scale;
+    const float* scale;  // NULL, or [B][5] {gain, pad_x, pad_y, orig_w, orig_h} per image (b2_nms_scaled): replaces the scalars above
     float* out; int32_t* out_count; int32_t* out_idx;
     unsigned long long* ws_keys; int32_t* ws_pay; float4* ws_box; int P_max;
     int debug;          // B2_NMS_DEBUG=1: thread 0 of every CTA leaves clock64() stamps of its phases in its ws_box slice (exact mode only)
@@ -321,6 +322,8 @@ __device__ __forceinline__ bool iou_exceeds(const float4 bi, const float area_i,
     return __fdiv_rn(inter, __fsub_rn(__fadd_rn(area_i, area_j), inter)) > thr;
 }
 
+// kScaled: the epilogue reads image b's row of p.scale (b2_nms_scaled); the scalar instance is b2_nms
+template <bool kScaled>
 __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const NmsParams p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
     unsigned long long* const s_keys = reinterpret_cast<unsigned long long*>(s_raw);          // [kSmemSort]
@@ -550,7 +553,14 @@ __global__ void __launch_bounds__(kNmsThreads, 1) nms_kernel(const NmsParams p) 
         const int src = pay[s_keep[k]];
         const float* c = cand + (size_t)src * 6;
         float x1 = c[0], y1 = c[1], x2 = c[2], y2 = c[3];
-        if (p.do_scale) {
+        if (kScaled) {
+            const float* sc = p.scale + (size_t)b * 5;
+            const float gain = sc[0], pad_x = sc[1], pad_y = sc[2], orig_w = sc[3], orig_h = sc[4];
+            x1 = __fdiv_rn(__fsub_rn(x1, pad_x), gain); y1 = __fdiv_rn(__fsub_rn(y1, pad_y), gain);
+            x2 = __fdiv_rn(__fsub_rn(x2, pad_x), gain); y2 = __fdiv_rn(__fsub_rn(y2, pad_y), gain);
+            x1 = fminf(fmaxf(x1, 0.f), orig_w); x2 = fminf(fmaxf(x2, 0.f), orig_w);
+            y1 = fminf(fmaxf(y1, 0.f), orig_h); y2 = fminf(fmaxf(y2, 0.f), orig_h);
+        } else if (p.do_scale) {
             x1 = __fdiv_rn(__fsub_rn(x1, p.pad_x), p.gain); y1 = __fdiv_rn(__fsub_rn(y1, p.pad_y), p.gain);
             x2 = __fdiv_rn(__fsub_rn(x2, p.pad_x), p.gain); y2 = __fdiv_rn(__fsub_rn(y2, p.pad_y), p.gain);
             x1 = fminf(fmaxf(x1, 0.f), p.orig_w); x2 = fminf(fmaxf(x2, 0.f), p.orig_w);
@@ -648,9 +658,9 @@ extern "C" size_t b2_nms_workspace_bytes(int B, int cand_cap) {
     return (size_t)B * (P * (8 + 4 + 16)) + 256;
 }
 
-extern "C" int b2_nms(const float* cand, const int32_t* cand_idx, const int32_t* cand_count, int cand_cap, int B,
+static int launch_nms(const float* cand, const int32_t* cand_idx, const int32_t* cand_count, int cand_cap, int B,
                       float iou_thres, int max_det, int max_nms, int agnostic, float max_wh, int mode,
-                      float gain, float pad_x, float pad_y, float orig_w, float orig_h, int do_scale,
+                      float gain, float pad_x, float pad_y, float orig_w, float orig_h, int do_scale, const float* scale,
                       float* out, int32_t* out_count, int32_t* out_idx, void* workspace, size_t workspace_bytes, void* stream) {
     B2_REQUIRE(cand && cand_idx && cand_count && out && out_count && workspace, "nms: null pointer");
     B2_REQUIRE(max_det >= 1 && max_det <= kMaxKeep, "nms: max_det=%d out of range [1,%d]", max_det, kMaxKeep);
@@ -664,7 +674,7 @@ extern "C" int b2_nms(const float* cand, const int32_t* cand_idx, const int32_t*
     NmsParams p{};
     p.cand = cand; p.cand_idx = cand_idx; p.cand_count = cand_count; p.cand_cap = cand_cap; p.B = B;
     p.iou_thres = iou_thres; p.max_det = max_det; p.max_nms = max_nms; p.agnostic = agnostic; p.max_wh = max_wh; p.mode = mode;
-    p.gain = gain; p.pad_x = pad_x; p.pad_y = pad_y; p.orig_w = orig_w; p.orig_h = orig_h; p.do_scale = do_scale;
+    p.gain = gain; p.pad_x = pad_x; p.pad_y = pad_y; p.orig_w = orig_w; p.orig_h = orig_h; p.do_scale = do_scale; p.scale = scale;
     p.out = out; p.out_count = out_count; p.out_idx = out_idx;
     const size_t P = (size_t)next_pow2(cand_cap);
     char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
@@ -675,9 +685,26 @@ extern "C" int b2_nms(const float* cand, const int32_t* cand_idx, const int32_t*
     { static const bool dbg = [] { const char* v = getenv("B2_NMS_DEBUG"); return v && atoi(v) != 0; }(); p.debug = dbg ? 1 : 0; }
     const size_t dyn = (size_t)kSmemSort * 12 + (size_t)kFastN * 16 + (size_t)kFastN * ((kFastN + 31) / 32) * 4 + (size_t)kMaxKeep * 16;
     // the attribute belongs to the current device's context: set on every call (a microsecond of host time), not once per process
-    B2_CUDA(cudaFuncSetAttribute(nms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    nms_kernel<<<B, kNmsThreads, dyn, (cudaStream_t)stream>>>(p);
+    auto kernel = scale ? nms_kernel<true> : nms_kernel<false>;
+    B2_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    kernel<<<B, kNmsThreads, dyn, (cudaStream_t)stream>>>(p);
     B2_CUDA(cudaGetLastError());
     b2_count_launch(1);
     return B2_OK;
+}
+
+extern "C" int b2_nms(const float* cand, const int32_t* cand_idx, const int32_t* cand_count, int cand_cap, int B,
+                      float iou_thres, int max_det, int max_nms, int agnostic, float max_wh, int mode,
+                      float gain, float pad_x, float pad_y, float orig_w, float orig_h, int do_scale,
+                      float* out, int32_t* out_count, int32_t* out_idx, void* workspace, size_t workspace_bytes, void* stream) {
+    return launch_nms(cand, cand_idx, cand_count, cand_cap, B, iou_thres, max_det, max_nms, agnostic, max_wh, mode,
+                      gain, pad_x, pad_y, orig_w, orig_h, do_scale, nullptr, out, out_count, out_idx, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b2_nms_scaled(const float* cand, const int32_t* cand_idx, const int32_t* cand_count, int cand_cap, int B,
+                             float iou_thres, int max_det, int max_nms, int agnostic, float max_wh, int mode, const float* scale,
+                             float* out, int32_t* out_count, int32_t* out_idx, void* workspace, size_t workspace_bytes, void* stream) {
+    B2_REQUIRE(scale, "nms_scaled: null scale table");
+    return launch_nms(cand, cand_idx, cand_count, cand_cap, B, iou_thres, max_det, max_nms, agnostic, max_wh, mode,
+                      1.f, 0.f, 0.f, 0.f, 0.f, 0, scale, out, out_count, out_idx, workspace, workspace_bytes, stream);
 }

@@ -403,32 +403,133 @@ __global__ void __launch_bounds__(256) preprocess_u8_kernel(const uint8_t* __res
 // cv2.resize(INTER_LINEAR) for uint8, bit-exact: 11-bit fixed-point coefficients (INTER_RESIZE_COEF_BITS = 11),
 // coefficients rounded with saturate_cast<short>(rint(f * 2048)), vertical pass result
 // (x >> 4 * beta >> 16 ...) reproduced with the 8u formula  ((b0*(S0>>4))>>16 + (b1*(S1>>4))>>16 + 2) >> 2.
+// The three functions below are the only copy of that arithmetic; every resize kernel samples through them.
+struct CvTap { int i0, i1, w0, w1; };      // source indices and their 11-bit weights for one destination index
+
+// cv::resize: f = (float)((d + 0.5) * scale - 0.5) in double, rounded once -- no fused multiply-add.  scale = 1 / (dst / src).
+// Horizontal taps: an index outside [0, n-1) is clamped AND its fraction zeroed (the xofs / alpha tables of cv::resize).
+__device__ __forceinline__ CvTap cv_tap_x(int d, double scale, int n) {
+    float f = (float)__dsub_rn(__dmul_rn((double)d + 0.5, scale), 0.5);
+    int s = (int)floorf(f); f -= s;
+    if (s < 0) { f = 0; s = 0; }
+    if (s >= n - 1) { f = 0; s = n - 1; }
+    return {s, min(s + 1, n - 1), __float2int_rn((1.f - f) * 2048.f), __float2int_rn(f * 2048.f)};
+}
+
+// Vertical taps: the two row indices are clamped, the fraction is kept (yofs / beta).
+__device__ __forceinline__ CvTap cv_tap_y(int d, double scale, int n) {
+    float f = (float)__dsub_rn(__dmul_rn((double)d + 0.5, scale), 0.5);
+    const int s = (int)floorf(f); f -= s;
+    return {min(max(s, 0), n - 1), min(max(s + 1, 0), n - 1), __float2int_rn((1.f - f) * 2048.f), __float2int_rn(f * 2048.f)};
+}
+
+// One output byte from the 2 x 2 neighbourhood (p_row_col) of one channel.
+__device__ __forceinline__ int cv_sample_u8(int p00, int p01, int p10, int p11, int a0, int a1, int b0, int b1) {
+    const int S0 = p00 * a0 + p01 * a1;
+    const int S1 = p10 * a0 + p11 * a1;
+    const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
+    return min(max(v, 0), 255);
+}
+
 __global__ void __launch_bounds__(256) resize_bilinear_u8_kernel(const uint8_t* __restrict__ src, int B, int sh, int sw,
                                                                  uint8_t* __restrict__ dst, int dh, int dw, double fy, double fx) {
     const size_t total = (size_t)B * dh * dw;
     const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
     const int x = (int)(idx % dw), y = (int)((idx / dw) % dh), b = (int)(idx / ((size_t)dw * dh));
-    // cv::resize: fx = (float)((dx + 0.5) * scale_x - 0.5) in double, rounded once -- no fused multiply-add
-    float sxf = (float)__dsub_rn(__dmul_rn((double)x + 0.5, fx), 0.5);
-    int sx = (int)floorf(sxf); sxf -= sx;
-    if (sx < 0) { sxf = 0; sx = 0; }
-    if (sx >= sw - 1) { sxf = 0; sx = sw - 1; }
-    float syf = (float)__dsub_rn(__dmul_rn((double)y + 0.5, fy), 0.5);
-    int sy = (int)floorf(syf); syf -= sy;
-    int sy0 = min(max(sy, 0), sh - 1), sy1 = min(max(sy + 1, 0), sh - 1);
-    const int a0 = __float2int_rn((1.f - sxf) * 2048.f), a1 = __float2int_rn(sxf * 2048.f);
-    const int b0 = __float2int_rn((1.f - syf) * 2048.f), b1 = __float2int_rn(syf * 2048.f);
-    const int sx1 = min(sx + 1, sw - 1);
-    const uint8_t* r0 = src + ((size_t)b * sh + sy0) * sw * 3;
-    const uint8_t* r1 = src + ((size_t)b * sh + sy1) * sw * 3;
+    const CvTap tx = cv_tap_x(x, fx, sw), ty = cv_tap_y(y, fy, sh);
+    const uint8_t* r0 = src + ((size_t)b * sh + ty.i0) * sw * 3;
+    const uint8_t* r1 = src + ((size_t)b * sh + ty.i1) * sw * 3;
     uint8_t* o = dst + idx * 3;
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        const int S0 = r0[sx * 3 + c] * a0 + r0[sx1 * 3 + c] * a1;
-        const int S1 = r1[sx * 3 + c] * a0 + r1[sx1 * 3 + c] * a1;
-        const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
-        o[c] = (uint8_t)min(max(v, 0), 255);
+    for (int c = 0; c < 3; ++c)
+        o[c] = (uint8_t)cv_sample_u8(r0[tx.i0 * 3 + c], r0[tx.i1 * 3 + c], r1[tx.i0 * 3 + c], r1[tx.i1 * 3 + c], tx.w0, tx.w1, ty.w0, ty.w1);
+}
+
+// LetterBox (data/augment.py:1692-1733) for a ragged batch.  Grid (bands of canvas rows, image); a thread writes 16 canvas pixels
+// (48 bytes, three 16-byte stores: canvas rows are W*3 bytes with W % 16 == 0, so every group is 16-byte aligned).  Rows and
+// columns outside the placed image are 114 without a read.  A resized image shares its column taps across all its rows: the CTA
+// puts them in shared memory once, and the row taps of its band too.  An unresized image is copied (16-byte loads when aligned).
+constexpr int kLbThreads = 256;
+constexpr int kLbMaxW = 4096;        // column-tap table: 8 bytes per canvas column in static shared memory
+constexpr int kLbMaxBand = 64;
+
+__global__ void __launch_bounds__(kLbThreads) letterbox_u8_kernel(const uint8_t* __restrict__ src, const int64_t* __restrict__ src_off,
+                                                                  const int32_t* __restrict__ geom, int H, int W, int band,
+                                                                  uint8_t* __restrict__ canvas) {
+    __shared__ int2 s_col[kLbMaxW];            // {byte offset of tap 0, (tap 1 - tap 0 in bytes: 0 or 3) << 28 | w0 << 16 | w1}
+    __shared__ int4 s_row[kLbMaxBand];         // {row 0 byte offset, row 1 byte offset, b0, b1}
+    const int b = blockIdx.y, y0 = blockIdx.x * band, y1 = min(H, y0 + band);
+    const int* g = geom + (size_t)b * 6;
+    const int sh = g[0], sw = g[1], top = g[4], left = g[5];
+    int rh = g[2], rw = g[3];
+    // a placement that does not fit the canvas (or an empty source) leaves the whole canvas at 114 instead of writing out of bounds
+    if (sh <= 0 || sw <= 0 || top < 0 || left < 0 || rh < 0 || rw < 0 || top + rh > H || left + rw > W) rh = rw = 0;
+    const uint8_t* img = src + src_off[b];
+    const bool copy = rh == sh && rw == sw;
+    // 16-pixel groups all inside or all outside the image, on 16-byte source addresses
+    const bool copy16 = copy && left % 16 == 0 && sw % 16 == 0 && src_off[b] % 16 == 0;
+    if (!copy) {
+        const double fx = 1.0 / ((double)rw / sw), fy = 1.0 / ((double)rh / sh);     // scale = 1 / inv_scale as cv::resize forms it
+        for (int x = threadIdx.x; x < rw; x += kLbThreads) {
+            const CvTap t = cv_tap_x(x, fx, sw);
+            s_col[x] = make_int2(t.i0 * 3, ((t.i1 - t.i0) * 3) << 28 | t.w0 << 16 | t.w1);
+        }
+        for (int r = threadIdx.x; r < y1 - y0; r += kLbThreads) {
+            const int y = y0 + r - top;
+            if (y >= 0 && y < rh) {
+                const CvTap t = cv_tap_y(y, fy, sh);
+                s_row[r] = make_int4(t.i0 * sw * 3, t.i1 * sw * 3, t.w0, t.w1);
+            }
+        }
+        __syncthreads();
+    }
+    const int groups = W / 16;
+    uint8_t* out = canvas + (size_t)b * H * W * 3;
+    for (int it = threadIdx.x; it < (y1 - y0) * groups; it += kLbThreads) {
+        const int r = it / groups, gx = (it - r * groups) * 16, y = y0 + r, sy = y - top;
+        uint4* o = reinterpret_cast<uint4*>(out + ((size_t)y * W + gx) * 3);
+        const bool row_in = sy >= 0 && sy < rh;
+        if (!row_in || gx + 16 <= left || gx >= left + rw) {
+            const uint4 fill = make_uint4(0x72727272u, 0x72727272u, 0x72727272u, 0x72727272u);
+            o[0] = fill; o[1] = fill; o[2] = fill;
+            continue;
+        }
+        if (copy16) {
+            const uint4* s = reinterpret_cast<const uint4*>(img + ((size_t)sy * sw + (gx - left)) * 3);
+            o[0] = s[0]; o[1] = s[1]; o[2] = s[2];
+            continue;
+        }
+        uint32_t w[12];
+#pragma unroll
+        for (int k = 0; k < 12; ++k) w[k] = 0;
+        int4 rt = make_int4(sy * sw * 3, 0, 0, 0);
+        if (!copy) rt = s_row[r];
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+            const int x = gx + i - left;
+            int v0 = 114, v1 = 114, v2 = 114;
+            if (x >= 0 && x < rw) {
+                if (copy) {
+                    const uint8_t* p = img + rt.x + x * 3;
+                    v0 = p[0]; v1 = p[1]; v2 = p[2];
+                } else {
+                    const int2 c = s_col[x];
+                    const int a0 = (c.y >> 16) & 0xfff, a1 = c.y & 0xffff, d = c.y >> 28;
+                    const uint8_t* p0 = img + rt.x + c.x;
+                    const uint8_t* p1 = img + rt.y + c.x;
+                    v0 = cv_sample_u8(p0[0], p0[d], p1[0], p1[d], a0, a1, rt.z, rt.w);
+                    v1 = cv_sample_u8(p0[1], p0[d + 1], p1[1], p1[d + 1], a0, a1, rt.z, rt.w);
+                    v2 = cv_sample_u8(p0[2], p0[d + 2], p1[2], p1[d + 2], a0, a1, rt.z, rt.w);
+                }
+            }
+            w[(3 * i) / 4] |= (uint32_t)v0 << (8 * ((3 * i) % 4));
+            w[(3 * i + 1) / 4] |= (uint32_t)v1 << (8 * ((3 * i + 1) % 4));
+            w[(3 * i + 2) / 4] |= (uint32_t)v2 << (8 * ((3 * i + 2) % 4));
+        }
+        o[0] = make_uint4(w[0], w[1], w[2], w[3]);
+        o[1] = make_uint4(w[4], w[5], w[6], w[7]);
+        o[2] = make_uint4(w[8], w[9], w[10], w[11]);
     }
 }
 
@@ -496,6 +597,21 @@ extern "C" int b2_resize_bilinear_u8(const uint8_t* src, int B, int sh, int sw, 
     const size_t total = (size_t)B * dh * dw;
     resize_bilinear_u8_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         src, B, sh, sw, dst, dh, dw, 1.0 / ((double)dh / sh), 1.0 / ((double)dw / sw));   // scale = 1 / inv_scale as cv::resize forms it
+    B2_CUDA(cudaGetLastError());
+    b2_count_launch(1);
+    return B2_OK;
+}
+
+extern "C" int b2_letterbox_u8(const uint8_t* src, const int64_t* src_off, const int32_t* geom, int B, int H, int W, uint8_t* canvas,
+                               void* stream) {
+    B2_REQUIRE(src && src_off && geom && canvas, "letterbox: null pointer");
+    B2_REQUIRE(B >= 1 && B <= 65535 && H >= 1, "letterbox: bad batch %d / height %d", B, H);
+    B2_REQUIRE(W >= 16 && W <= kLbMaxW && W % 16 == 0, "letterbox: canvas width %d must be a multiple of 16 in [16, %d]", W, kLbMaxW);
+    B2_REQUIRE((uintptr_t)src % 16 == 0 && (uintptr_t)canvas % 16 == 0, "letterbox: source and canvas must be 16-byte aligned");
+    // a band of rows per CTA: about four 16-pixel groups per thread, so the tap tables are amortised over enough work
+    const int band = min(kLbMaxBand, max(1, 4 * kLbThreads / (W / 16)));
+    letterbox_u8_kernel<<<dim3((unsigned)b2_ceil_div(H, band), (unsigned)B), kLbThreads, 0, (cudaStream_t)stream>>>(
+        src, src_off, geom, H, W, band, canvas);
     B2_CUDA(cudaGetLastError());
     b2_count_launch(1);
     return B2_OK;

@@ -2,6 +2,7 @@
 
   conv2d_bf16            Conv.forward_fuse (ultralytics/nn/modules/conv.py:83-93) on NHWC bf16 tensors
   sppf_pool, upsample_slice, stem_u8, preprocess_u8, resize_bilinear_u8
+  letterbox_u8           LetterBox (data/augment.py:1692-1733) of a ragged batch packed by ``pack_frames``
   decode                 Detect._inference (ultralytics/nn/modules/head.py:152-187) + candidate filter
   nms                    tail of non_max_suppression (ultralytics/utils/nms.py:129-160) + scale_boxes
   non_max_suppression    the reference signature (ultralytics/utils/nms.py:13-167) on a (B, 4+nc, A) tensor
@@ -128,6 +129,46 @@ def resize_bilinear_u8(frames, dh, dw, stream=None):
     return out
 
 
+def pack_layout(shapes):
+    """Byte offsets (int64 [B], each a multiple of 16) of HWC uint8 frames of ``shapes`` [(h, w), ...] packed back to back, and the
+    packed size.  16-byte offsets let ``letterbox_u8`` copy unresized frames with vector loads."""
+    offs, n = [], 0
+    for h, w in shapes:
+        offs.append(n)
+        n += -(-int(h) * int(w) * 3 // 16) * 16
+    return np.asarray(offs, np.int64), n
+
+
+def pack_frames(frames, out=None):
+    """Pack HWC BGR uint8 frames at the offsets of :func:`pack_layout` into ``out`` (a 1-D uint8 numpy array or CPU tensor,
+    e.g. pinned; a new array when None).  Returns (packed, offsets)."""
+    offs, n = pack_layout([f.shape[:2] for f in frames])
+    if out is None:
+        out = np.empty((n,), np.uint8)
+    buf = out.numpy() if hasattr(out, "numpy") else out
+    if buf.ndim != 1 or buf.dtype != np.uint8 or buf.shape[0] != n:
+        raise ValueError(f"packed buffer: need {n} uint8 bytes, got {buf.dtype} {tuple(buf.shape)}")
+    for f, o in zip(frames, offs):
+        if not (f.ndim == 3 and f.shape[2] == 3 and f.dtype == np.uint8):
+            raise TypeError("frames must be HWC BGR uint8 arrays")
+        buf[o:o + f.size] = np.ascontiguousarray(f).reshape(-1)
+    return out, offs
+
+
+def letterbox_u8(packed, offsets, geom, H, W, out=None, stream=None):
+    """LetterBox of a ragged batch: ``packed`` CUDA uint8 (frames at ``offsets``, CUDA int64 [B]), ``geom`` CUDA int32 [B][6]
+    {src_h, src_w, rh, rw, top, left} (``predictor.letterbox_table``).  Returns (or fills) the canvas [B][H][W][3] uint8."""
+    torch = _torch()
+    lib = _lib.load()
+    B = geom.shape[0]
+    if out is None:
+        out = torch.empty((B, H, W, 3), dtype=torch.uint8, device=packed.device)
+    assert tuple(out.shape) == (B, H, W, 3) and out.is_contiguous() and packed.is_contiguous()
+    assert offsets.dtype == torch.int64 and geom.dtype == torch.int32 and offsets.shape[0] == B and tuple(geom.shape) == (B, 6)
+    _lib.check(lib.b2_letterbox_u8(_lib.ptr(packed), _lib.ptr(offsets), _lib.ptr(geom), B, H, W, _lib.ptr(out), _lib.stream_ptr(stream)))
+    return out
+
+
 def sppf_pool(buf, coff, c, stream=None):
     lib = _lib.load()
     B, H, W, cs = buf.shape
@@ -184,7 +225,16 @@ class DetectPost:
                                                     _lib.stream_ptr(stream)))
 
     def nms(self, iou, agnostic=False, mode="exact", max_nms=MAX_NMS, scale=None, stream=None):
-        """scale: None or (gain, pad_x, pad_y, orig_w, orig_h) for the fused scale_boxes/clip_boxes epilogue."""
+        """scale: None or (gain, pad_x, pad_y, orig_w, orig_h) for the fused scale_boxes/clip_boxes epilogue, or a CUDA float32
+        [B][5] tensor of those per image (frames of different original shapes)."""
+        torch = _torch()
+        if isinstance(scale, torch.Tensor):
+            assert scale.is_cuda and scale.dtype == torch.float32 and tuple(scale.shape) == (self.B, 5) and scale.is_contiguous()
+            _lib.check(self.lib.b2_nms_scaled(_lib.ptr(self.cand), _lib.ptr(self.cand_idx), _lib.ptr(self.cand_count), self.cand_cap, self.B,
+                                              float(iou), self.max_det, int(max_nms), int(bool(agnostic)), MAX_WH, {"exact": 0, "legacy": 1}[mode],
+                                              _lib.ptr(scale), _lib.ptr(self.out), _lib.ptr(self.out_count), _lib.ptr(self.out_idx),
+                                              _lib.ptr(self.ws), self.ws_bytes, _lib.stream_ptr(stream)))
+            return self.out, self.out_count
         g = scale or (1.0, 0.0, 0.0, 0.0, 0.0)
         _lib.check(self.lib.b2_nms(_lib.ptr(self.cand), _lib.ptr(self.cand_idx), _lib.ptr(self.cand_count), self.cand_cap, self.B,
                                    float(iou), self.max_det, int(max_nms), int(bool(agnostic)), MAX_WH, {"exact": 0, "legacy": 1}[mode],

@@ -13,8 +13,8 @@ execution shards streams across ranks with no collective on the data path; NCCL 
 """
 from __future__ import annotations
 
-from . import _lib, cfg, weights
-from .predictor import DetectPipeline, letterbox_geometry
+from . import _lib, cfg, ops, weights
+from .predictor import DetectPipeline, letterbox_table
 from .tracker import TrackerBank
 
 
@@ -57,18 +57,28 @@ class DetectTrackPipeline:
         capacity: track slots per stream.  The reference's track list is unbounded; ``results()`` raises if a detection was
         ever dropped for lack of a slot and grows the bank (x2) once a stream uses more than half of it.
         max_tracks_out: rows per stream of the result block (default: capacity).  The download moves exactly this block,
-        so a caller that expects tens of tracks per stream keeps it small; ``results()`` raises if a stream reported more."""
+        so a caller that expects tens of tracks per stream keeps it small; ``results()`` raises if a stream reported more.
+        frame_hw: the (h, w) of every stream, or a list of S shapes, one per stream (fixed for the pipeline's life).  Streams that
+        all share one shape needing no resize take the frames as [S][h][w][3] and letterbox inside the stem kernel.  Any other
+        set of shapes (mixed, or one shape that needs a resize) is the general path: frames are packed back to back
+        (``ops.pack_frames``), letterboxed on the GPU into one canvas -- ``auto`` padding for one common shape, the full imgsz
+        canvas for mixed shapes, as YOLO.predict does -- and NMS scales each stream's boxes to its own frame."""
         import torch
 
         self.device = _lib.require_cuda()
         self.spec = cfg.resolve(model, nc=nc)
         sd = weights.to_numpy_state_dict(state_dict) if state_dict is not None else weights.synthetic_state_dict(self.spec, seed)
         self.S = int(n_streams)
-        self.h0, self.w0 = frame_hw
+        shapes = [tuple(hw) for hw in frame_hw] if hasattr(frame_hw[0], "__len__") else [tuple(frame_hw)] * self.S
+        if len(shapes) != self.S:
+            raise ValueError(f"frame_hw lists {len(shapes)} shapes for {self.S} streams")
+        self.frame_shapes = [(int(h), int(w)) for h, w in shapes]
         isz = [imgsz, imgsz] if isinstance(imgsz, int) else list(imgsz)
-        (rh, rw), (self.H, self.W), self.top, self.left = letterbox_geometry(self.h0, self.w0, isz, auto=True)
-        if (rh, rw) != (self.h0, self.w0):
-            raise NotImplementedError("pipeline frames must not need a resize (use YOLO.predict for the general letterbox)")
+        (self.H, self.W), geom, scale = letterbox_table(self.frame_shapes, isz)
+        # identity letterbox (every stream one shape, no resize): the stem kernel pads the frames itself
+        self.ragged = len(set(self.frame_shapes)) != 1 or tuple(geom[0, 2:4]) != self.frame_shapes[0]
+        self.h0, self.w0 = self.frame_shapes[0]
+        self.top, self.left = int(geom[0, 4]), int(geom[0, 5])
         self.conf, self.iou, self.nms_mode = float(conf), float(iou), nms_mode
         self.detect = DetectPipeline(self.spec, sd, self.S, self.H, self.W, max_det)
         self.max_det = int(max_det)
@@ -78,7 +88,12 @@ class DetectTrackPipeline:
         self.flops_per_frame = self.detect.engine.flops_per_image
         # double-buffered staging for the host-facing path
         self._copy_stream = torch.cuda.Stream()
-        self._dev_frames = [torch.empty((self.S, self.h0, self.w0, 3), dtype=torch.uint8, device=self.device) for _ in range(2)]
+        if self.ragged:
+            offs, self.packed_bytes = ops.pack_layout(self.frame_shapes)
+            self._offsets, self._geom, self._scale = (torch.from_numpy(a).to(self.device) for a in (offs, geom, scale))
+            self._dev_frames = [torch.empty((self.packed_bytes,), dtype=torch.uint8, device=self.device) for _ in range(2)]
+        else:
+            self._dev_frames = [torch.empty((self.S, self.h0, self.w0, 3), dtype=torch.uint8, device=self.device) for _ in range(2)]
         self._ready = [torch.cuda.Event() for _ in range(2)]
         self._consumed = [torch.cuda.Event() for _ in range(2)]
         self._slot = 0
@@ -92,7 +107,7 @@ class DetectTrackPipeline:
         self._step_done = torch.cuda.Event()
         self._rows_downloaded = torch.cuda.Event()
         self._rows_downloaded.record()
-        self.h2d_bytes_per_step = self.S * self.h0 * self.w0 * 3
+        self.h2d_bytes_per_step = self._dev_frames[0].numel()
         self._alloc_host()
 
     def _alloc_host(self):
@@ -103,22 +118,38 @@ class DetectTrackPipeline:
         self.host_stats = torch.zeros((self.S, 8), dtype=torch.int64).pin_memory()
         self.d2h_bytes_per_step = self.host_rows.numel() * 4 + self.host_counts.numel() * 4 + self.host_stats.numel() * 8
 
+    def _packed(self, frames):
+        """The general path's input: ``packed_bytes`` uint8 in the ``ops.pack_frames`` layout (any shape with that many bytes,
+        e.g. [S][h][w][3] when every frame is a multiple of 16 bytes)."""
+        if frames.dtype.itemsize != 1 or frames.numel() != self.packed_bytes or not frames.is_contiguous():
+            raise ValueError(f"expected {self.packed_bytes} contiguous packed frame bytes (ops.pack_frames of shapes {self.frame_shapes}), "
+                             f"got {frames.dtype} {tuple(frames.shape)}")
+        return frames.view(-1)
+
     def step_device(self, frames_u8, with_trajectory=False, stream=None):
-        """frames_u8: CUDA uint8 [S][h][w][3] BGR.  Returns (track rows [S][capacity][20], counts [S]) on the GPU."""
+        """frames_u8: CUDA uint8 [S][h][w][3] BGR, or on the general path (mixed / resized shapes) the packed frames of
+        ``ops.pack_frames``.  Returns (track rows [S][capacity][20], counts [S]) on the GPU."""
         import torch
 
         cur = stream or torch.cuda.current_stream()
         if not self.overlap_post:
-            dets, counts = self.detect(frames_u8, self.conf, self.iou, self.top, self.left, (self.h0, self.w0), None, False,
-                                       self.nms_mode, stream)
+            if self.ragged:
+                dets, counts = self.detect.run_ragged(self._packed(frames_u8), self._offsets, self._geom, self._scale, self.conf, self.iou,
+                                                      None, False, self.nms_mode, stream)
+            else:
+                dets, counts = self.detect(frames_u8, self.conf, self.iou, self.top, self.left, (self.h0, self.w0), None, False,
+                                           self.nms_mode, stream)
             # the bank's row block is about to be rewritten: a download of the previous step's rows (step_host) must be over
             cur.wait_event(self._rows_downloaded)
             return self.bank.update(dets, counts, with_trajectory=with_trajectory, stream=stream)
         d, ps = self.detect, self._post_stream
+        if self.ragged:
+            frames_u8 = d.letterbox(self._packed(frames_u8), self._offsets, self._geom, stream)
         if self.forward_events is not None:           # bench.py: CUDA events around the forward graph, on the stream it runs on
             ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
             ev[0].record(cur)
-        d.engine.forward_u8(frames_u8, self.top, self.left, stream=stream)
+        top, left = (0, 0) if self.ragged else (self.top, self.left)
+        d.engine.forward_u8(frames_u8, top, left, stream=stream)
         if self.forward_events is not None:
             ev[1].record(cur)
             self.forward_events.append(ev)
@@ -127,14 +158,17 @@ class DetectTrackPipeline:
         self._cand_done.record(cur)
         ps.wait_event(self._cand_done)
         ps.wait_event(self._rows_downloaded)
-        dets, counts = d.nms(self.iou, (self.h0, self.w0), False, self.nms_mode, ps)
+        if self.ragged:
+            dets, counts = d.nms(self.iou, None, False, self.nms_mode, ps, self._scale)
+        else:
+            dets, counts = d.nms(self.iou, (self.h0, self.w0), False, self.nms_mode, ps)
         out = self.bank.update(dets, counts, with_trajectory=with_trajectory, stream=ps)
         self._post_done.record(ps)
         return out
 
     def step_host(self, frames_pinned):
-        """frames_pinned: pinned host uint8 [S][h][w][3].  Upload on the copy stream (overlaps the previous step's
-        compute), run the step, download rows + counts into pinned host buffers on a third stream (overlaps the next
+        """frames_pinned: pinned host uint8 [S][h][w][3] (general path: the ``ops.pack_frames`` buffer).  Upload on the copy
+        stream (overlaps the previous step's compute), run the step, download rows + counts into pinned host buffers on a third stream (overlaps the next
         step).  Returns the host buffers (valid after ``join()`` + ``torch.cuda.current_stream().synchronize()``)."""
         import torch
 
@@ -143,7 +177,7 @@ class DetectTrackPipeline:
         self._slot ^= 1
         with torch.cuda.stream(self._copy_stream):
             self._copy_stream.wait_event(self._consumed[k])          # the step that last read this buffer is done
-            self._dev_frames[k].copy_(frames_pinned, non_blocking=True)
+            self._dev_frames[k].copy_(self._packed(frames_pinned) if self.ragged else frames_pinned, non_blocking=True)
             self._ready[k].record(self._copy_stream)
         cur.wait_event(self._ready[k])
         rows, counts = self.step_device(self._dev_frames[k])
@@ -178,14 +212,14 @@ class DetectTrackPipeline:
         import numpy as np
         import torch
 
-        stage = torch.empty((self.S, self.h0, self.w0, 3), dtype=torch.uint8).pin_memory()
+        stage = torch.empty(tuple(self._dev_frames[0].shape), dtype=torch.uint8).pin_memory()
         for sources, frames, _ in loader:
-            if len(frames) != self.S:
-                raise ValueError(f"the loader delivered {len(frames)} frames, the pipeline was built for {self.S} streams")
-            for k, f in enumerate(frames):
-                if f.shape != (self.h0, self.w0, 3):
-                    raise ValueError(f"stream {k}: frame shape {f.shape}, the pipeline was built for {(self.h0, self.w0, 3)}")
-                stage[k] = torch.from_numpy(np.ascontiguousarray(f))
+            check_frames(frames, self.frame_shapes)
+            if self.ragged:
+                ops.pack_frames(frames, out=stage)
+            else:
+                for k, f in enumerate(frames):
+                    stage[k] = torch.from_numpy(np.ascontiguousarray(f))
             self.step_host(stage)
             rows, counts = self.results()                 # synchronises: `stage` may be refilled afterwards
             yield sources, rows.numpy().copy(), counts.numpy().copy()
@@ -203,6 +237,15 @@ class DetectTrackPipeline:
             if not self._fixed_out:
                 self._alloc_host()
         return self.host_rows, self.host_counts
+
+
+def check_frames(frames, shapes):
+    """Raises ValueError unless ``frames`` holds one HWC frame per stream, frame k of shape ``shapes[k]`` + (3,)."""
+    if len(frames) != len(shapes):
+        raise ValueError(f"the loader delivered {len(frames)} frames, the pipeline was built for {len(shapes)} streams")
+    for k, (f, hw) in enumerate(zip(frames, shapes)):
+        if tuple(f.shape) != (*hw, 3):
+            raise ValueError(f"stream {k}: frame shape {tuple(f.shape)}, the pipeline was built for {(*hw, 3)}")
 
 
 def check_bank(stats, counts, capacity, max_out):

@@ -273,6 +273,23 @@ def scale_params(canvas_hw, orig_hw):
     return gain, pad_x, pad_y, orig_hw[1], orig_hw[0]
 
 
+def letterbox_table(shapes, imgsz):
+    """LetterBox of a batch of frames of ``shapes`` [(h, w), ...] as BasePredictor.pre_transform (engine/predictor.py) chooses it:
+    ``auto`` (minimal stride padding) only when every shape is the same, else every frame into the full ``imgsz`` canvas.
+    Returns (canvas (H, W), geom int32 [B][6] {h, w, rh, rw, top, left} for ``ops.letterbox_u8``, scale float32 [B][5] of
+    ``scale_params`` per frame for the NMS epilogue)."""
+    shapes = [(int(h), int(w)) for h, w in shapes]
+    auto = len(set(shapes)) == 1
+    geom, scale, canvas = [], [], set()
+    for h0, w0 in shapes:
+        (rh, rw), hw, top, left = letterbox_geometry(h0, w0, imgsz, auto)
+        canvas.add(hw)
+        geom.append((h0, w0, rh, rw, top, left))
+        scale.append(scale_params(hw, (h0, w0)))
+    (H, W), = canvas
+    return (H, W), np.asarray(geom, np.int32).reshape(-1, 6), np.asarray(scale, np.float32).reshape(-1, 5)
+
+
 # ---------------------------------------------------------------------------------------------------
 # model facade
 # ---------------------------------------------------------------------------------------------------
@@ -285,6 +302,7 @@ class DetectPipeline:
         self.post = ops.DetectPost(batch, e.level_h, e.level_w, e.level_stride, e.nc, e.lstride, max_det=max_det)
         self.B, self.H, self.W = batch, H, W
         self.feats = None
+        self.canvas = None          # [B][H][W][3] uint8, allocated by the first ``letterbox``
 
     def __call__(self, frames_u8, conf, iou, pad_top=0, pad_left=0, orig_hw=None, classes_mask=None, agnostic=False,
                  mode="exact", stream=None):
@@ -296,9 +314,25 @@ class DetectPipeline:
         self.engine.forward_tensor(x, stream=stream)
         return self.finish(conf, iou, orig_hw, classes_mask, agnostic, mode, stream)
 
-    def finish(self, conf, iou, orig_hw, classes_mask, agnostic, mode, stream):
+    def letterbox(self, packed, offsets, geom, stream=None):
+        """LetterBox frames of individual shapes (``ops.pack_frames`` layout, CUDA tables of ``letterbox_table``) into
+        ``self.canvas``."""
+        import torch
+
+        if self.canvas is None:
+            self.canvas = torch.empty((self.B, self.H, self.W, 3), dtype=torch.uint8, device=packed.device)
+        return ops.letterbox_u8(packed, offsets, geom, self.H, self.W, out=self.canvas, stream=stream)
+
+    def run_ragged(self, packed, offsets, geom, scale, conf, iou, classes_mask=None, agnostic=False, mode="exact", stream=None):
+        """A batch of frames of individual shapes: letterbox, forward on the canvas, candidates, NMS with each image's
+        scale_boxes (``scale``: CUDA float32 [B][5]).  Returns (dets [B][max_det][6], counts [B]) like ``__call__``."""
+        self.letterbox(packed, offsets, geom, stream)
+        self.engine.forward_u8(self.canvas, 0, 0, stream=stream)
+        return self.finish(conf, iou, None, classes_mask, agnostic, mode, stream, scale)
+
+    def finish(self, conf, iou, orig_hw, classes_mask, agnostic, mode, stream, scale=None):
         self.candidates(conf, classes_mask, stream)
-        return self.nms(iou, orig_hw, agnostic, mode, stream)
+        return self.nms(iou, orig_hw, agnostic, mode, stream, scale)
 
     def candidates(self, conf, classes_mask=None, stream=None):
         """Head outputs -> per-image candidate lists (the only post-processing launch that reads engine buffers)."""
@@ -307,8 +341,10 @@ class DetectPipeline:
         else:
             self.post.decode(self.engine.level_ptrs, conf, classes_mask, stream=stream)
 
-    def nms(self, iou, orig_hw=None, agnostic=False, mode="exact", stream=None):
-        scale = scale_params((self.H, self.W), orig_hw) if orig_hw is not None else None
+    def nms(self, iou, orig_hw=None, agnostic=False, mode="exact", stream=None, scale=None):
+        """scale_boxes to ``orig_hw`` (one shape for the batch), or per image with ``scale`` (CUDA float32 [B][5])."""
+        if scale is None and orig_hw is not None:
+            scale = scale_params((self.H, self.W), orig_hw)
         return self.post.nms(iou, agnostic=agnostic, mode=mode, scale=scale, stream=stream)
 
     def embed(self, stream=None):
@@ -439,29 +475,32 @@ class YOLO:
             for f in frames:
                 if not (isinstance(f, np.ndarray) and f.ndim == 3 and f.shape[2] == 3 and f.dtype == np.uint8):
                     raise TypeError("source must be HWC BGR uint8 ndarray(s) or a BCHW float tensor")
-            same = len({f.shape for f in frames}) == 1
-            groups = [list(range(len(frames)))] if same else [[i] for i in range(len(frames))]
-            out = [None] * len(frames)
-            for idxs in groups:
-                h0, w0 = frames[idxs[0]].shape[:2]
-                t0 = time.perf_counter()
-                (rh, rw), (H, W), top, left = letterbox_geometry(h0, w0, imgsz, auto=same)
-                batch = torch.from_numpy(np.ascontiguousarray(np.stack([frames[i] for i in idxs]))).to(dev, non_blocking=True)
+            t0 = time.perf_counter()
+            if len({f.shape for f in frames}) == 1:
+                h0, w0 = frames[0].shape[:2]
+                (rh, rw), (H, W), top, left = letterbox_geometry(h0, w0, imgsz, auto=True)
+                batch = torch.from_numpy(np.ascontiguousarray(np.stack(frames))).to(dev, non_blocking=True)
                 if (rh, rw) != (h0, w0):
                     batch = ops.resize_bilinear_u8(batch, rh, rw)
-                if H % 32 or W % 32:           # auto=False canvases are imgsz, already stride multiples
+                if H % 32 or W % 32:
                     raise ValueError(f"letterboxed size {H}x{W} is not a multiple of 32")
-                pipe = self._pipe(len(idxs), H, W, max_det)
+                pipe = self._pipe(len(frames), H, W, max_det)
                 dets, counts = pipe(batch, conf, iou, top, left, (h0, w0), cmask, a["agnostic_nms"], a["nms_mode"])
-                feats = pipe.embed() if want_feats else None          # before the next group's forward reuses the arena
-                cnt = counts.cpu().tolist()
-                ms = (time.perf_counter() - t0) * 1e3 / len(idxs)
-                for j, i in enumerate(idxs):
-                    out[i] = Results(frames[i], f"image{i}.jpg", self.names, dets[j, :cnt[j]].clone(),
-                                     {"preprocess": 0.0, "inference": ms, "postprocess": 0.0})
-                    if want_feats:
-                        out[i].feats = feats[j, :cnt[j]].clone()
-            results = out
+            else:
+                # frames of different shapes: each letterboxed into the imgsz canvas (auto=False), all in one forward
+                (H, W), geom, scale = letterbox_table([f.shape[:2] for f in frames], imgsz)
+                packed, offs = ops.pack_frames(frames)
+                up = lambda arr: torch.from_numpy(arr).to(dev)
+                pipe = self._pipe(len(frames), H, W, max_det)
+                dets, counts = pipe.run_ragged(up(packed), up(offs), up(geom), up(scale), conf, iou, cmask, a["agnostic_nms"], a["nms_mode"])
+            feats = pipe.embed() if want_feats else None
+            cnt = counts.cpu().tolist()
+            ms = (time.perf_counter() - t0) * 1e3 / len(frames)
+            for i, f in enumerate(frames):
+                results.append(Results(f, f"image{i}.jpg", self.names, dets[i, :cnt[i]].clone(),
+                                       {"preprocess": 0.0, "inference": ms, "postprocess": 0.0}))
+                if want_feats:
+                    results[-1].feats = feats[i, :cnt[i]].clone()
         if a.get("verbose"):
             for r in results:
                 print(f"{r.orig_shape[0]}x{r.orig_shape[1]} {r.verbose()}{r.speed['inference']:.1f}ms")

@@ -41,7 +41,7 @@ def predictor_class():
     from ultralytics.models.yolo.detect import DetectionPredictor        # models/yolo/detect/predict.py:8
 
     from . import _lib, cfg, ops, weights
-    from .predictor import DetectPipeline, check_imgsz, letterbox_geometry
+    from .predictor import DetectPipeline, check_imgsz, letterbox_geometry, letterbox_table
 
     class B200DetectionPredictor(DetectionPredictor):
         """DetectionPredictor whose three stages run on the CUDA engine of this package (no Ultralytics module executes)."""
@@ -60,7 +60,8 @@ def predictor_class():
 
         def preprocess(self, im):
             """im: list of HWC BGR uint8 frames (LoadPilAndNumpy, data/loaders.py:519-558).  Uploads them; the letterbox border,
-            the channel swap and the /255 happen inside the stem kernel."""
+            the channel swap and the /255 happen inside the stem kernel.  Frames of different shapes (pre_transform's auto=False
+            case) are packed, uploaded once and letterboxed into the imgsz canvas on the GPU; NMS then scales boxes per frame."""
             import torch
 
             dev = _lib.require_cuda()                                  # raises without a CUDA device: there is no CPU fallback
@@ -68,25 +69,32 @@ def predictor_class():
                 raise NotImplementedError("tensor sources: use b200dt.predictor.YOLO.predict")
             frames = list(im)
             if len({f.shape for f in frames}) != 1:
-                raise NotImplementedError("frames of different shapes in one batch: predict them one at a time")
+                (H, W), geom, scale = letterbox_table([f.shape[:2] for f in frames], check_imgsz(self.imgsz))
+                packed, offs = ops.pack_frames(frames)
+                up = lambda arr: torch.from_numpy(arr).to(dev)
+                pipe = self._pipe_for(len(frames), H, W)
+                canvas = pipe.letterbox(up(packed), up(offs), up(geom))
+                self._b200_geom = (len(frames), H, W, 0, 0, None, up(scale))
+                return canvas
             h0, w0 = frames[0].shape[:2]
             (rh, rw), (H, W), top, left = letterbox_geometry(h0, w0, check_imgsz(self.imgsz), auto=True)
             u8 = torch.from_numpy(np.ascontiguousarray(np.stack(frames))).to(dev, non_blocking=True)
             if (rh, rw) != (h0, w0):
                 u8 = ops.resize_bilinear_u8(u8, rh, rw)
-            self._b200_geom = (len(frames), H, W, top, left, (h0, w0))
+            self._b200_geom = (len(frames), H, W, top, left, (h0, w0), None)
             return u8
 
         def inference(self, im, *args, **kwargs):
-            B, H, W, top, left, _ = self._b200_geom
+            B, H, W, top, left, _, _ = self._b200_geom
             self._pipe_for(B, H, W).engine.forward_u8(im, top, left)
             return im
 
         def postprocess(self, preds, img, orig_imgs, **kwargs):
-            B, H, W, _, _, orig_hw = self._b200_geom
+            B, H, W, _, _, orig_hw, scale = self._b200_geom
             pipe = self._pipe_for(B, H, W)
             cmask = ops._classes_mask(self.args.classes, len(self.model.names), img.device)
-            dets, counts = pipe.finish(float(self.args.conf), float(self.args.iou), orig_hw, cmask, bool(self.args.agnostic_nms), "exact", None)
+            dets, counts = pipe.finish(float(self.args.conf), float(self.args.iou), orig_hw, cmask, bool(self.args.agnostic_nms), "exact", None,
+                                       scale)
             n = counts.cpu().tolist()
             return results_from_dets([dets[i, :n[i]].clone() for i in range(B)], orig_imgs, self.batch[0], self.model.names)
 
