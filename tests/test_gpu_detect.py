@@ -39,87 +39,34 @@ def _diag(msg):
             fh.write(msg + "\n")
 
 
+@pytest.mark.parametrize("head", ["unfused", "fused", "fused-chain15"])
 @pytest.mark.parametrize("name,B,H,W", [("yolov8n-p2", 2, 64, 96), ("yolov8s-p2", 1, 96, 64), ("yolov8x-p2", 1, 64, 64), ("yolov8s-p2", 3, 128, 160),
                                         ("yolov8-small", 2, 64, 96)])      # the project's own model: widths 12 / 24 padded to 16 / 32
-def test_engine_every_layer_matches_oracle_on_identical_inputs(name, B, H, W):
-    """Primary kernel gate (SURVEY.md H1 (i)): after one engine forward, EVERY launch of the plan is re-evaluated by
-    the oracle on the engine's own input buffer (bf16 values, bf16 weights, fp32 accumulate) and must agree with
-    the engine's output buffer to about one bf16 rounding."""
-    from b200dt import engine as eng_mod
+def test_engine_every_layer_matches_oracle_on_identical_inputs(name, B, H, W, head, monkeypatch):
+    """Primary kernel gate (SURVEY.md H1 (i)): after one engine forward, EVERY launch of the plan is re-evaluated in float64
+    on the engine's own input buffer (bf16 values, bf16 weights) and must agree with the engine's output buffer to about one
+    bf16 rounding (tests/plan_ref.py).  ``fused``: the Detect head as DetectPipeline builds it, with the DFL and class-max
+    epilogues; ``fused-chain15`` (B2_CHAIN=15) also chains the class tail (conv_tc_kernel<2, 2, 2, 16, 1>)."""
     from b200dt.engine import Engine
 
+    import plan_ref
+
+    if head == "fused-chain15":
+        monkeypatch.setenv("B2_CHAIN", "15")
     torch = _torch()
     spec = cfg.resolve(name)
     sd = weights.synthetic_state_dict(spec, seed=0)
     x = pp.preprocess([synth.IRStream(seed=40 + b, h=H, w=W, n_targets=4).frame() for b in range(B)])
-    eng = Engine(spec, sd, B, H, W)
-    eng.forward_tensor(torch.from_numpy(x).cuda())
+    eng = Engine(spec, sd, B, H, W, fuse_head=head != "unfused")
+    xt = torch.from_numpy(x).cuda()
+    eng.forward_tensor(xt)
     torch.cuda.synchronize()
-    P = eng.plan
-    blob = P.blob.bytes()
-    bufs = {}
-
-    def buf(i):
-        if i not in bufs:
-            bufs[i] = eng.buffer(i).float().cpu().numpy()
-        return bufs[i]
-
-    worst = 0.0
-    for op in P.ops:
-        if op[0] == eng_mod.OP_CONV:
-            _, ib, ioff, cin, ob, ooff, cout, k, s, act, rb, roff, woff, boff = op[:14]
-            ib2, ioff2, cin2, up0, up1 = op[14:19]
-            xin = buf(ib)[..., ioff:ioff + cin]
-            if ib2 >= 0:                                            # folded Concat([Upsample(a), b])
-                x2 = buf(ib2)[..., ioff2:ioff2 + cin2]
-                xin = np.concatenate([xin.repeat(up0, 1).repeat(up0, 2), x2.repeat(up1, 1).repeat(up1, 2)], -1)
-                cin = cin + cin2
-            w = weights.bf16_bits_to_f32(np.frombuffer(blob, np.uint16, count=cout * k * k * cin, offset=woff)).reshape(cout, k, k, cin)
-            bias = np.frombuffer(blob, np.float32, count=cout, offset=boff)
-            xin = xin.transpose(0, 3, 1, 2)
-            ref = onet.conv2d(xin, np.ascontiguousarray(w.transpose(0, 3, 1, 2)), bias, s, k // 2)
-            if act:
-                ref = onet.silu(ref)
-            if rb >= 0:
-                ref = ref + buf(rb)[..., roff:roff + cout].transpose(0, 3, 1, 2)
-            if op[20]:
-                # chained 1x1 conv (engine.py, ConvParams::chain): the main conv's tile is rounded to bf16 (as the unchained
-                # path stores it), concatenated behind the extra source's channels, and fed to the 1x1 conv
-                w2off, b2off, cout2, act2, xb, xoff, xc = op[21:28]
-                mid = onet.bf16_round(ref)
-                if xb >= 0:
-                    mid = np.concatenate([buf(xb)[..., xoff:xoff + xc].transpose(0, 3, 1, 2), mid], 1)
-                k2 = cout + (xc if xb >= 0 else 0)
-                w2 = weights.bf16_bits_to_f32(np.frombuffer(blob, np.uint16, count=cout2 * k2, offset=w2off)).reshape(cout2, k2, 1, 1)
-                ref = onet.conv2d(mid, w2, np.frombuffer(blob, np.float32, count=cout2, offset=b2off), 1, 0)
-                if act2:
-                    ref = onet.silu(ref)
-                cout = cout2
-            got = buf(ob)[..., ooff:ooff + cout].transpose(0, 3, 1, 2)
-            err = _rel_l2(got, ref)
-            worst = max(worst, err)
-            assert err < 4e-3, (op, err)
-            np.testing.assert_allclose(got, ref, rtol=1e-2, atol=1e-2 * max(1.0, float(np.abs(ref).max()) / 16))
-        elif op[0] == eng_mod.OP_STEM:
-            _, ob, ooff, c0, woff, boff = op[:6]
-            w = weights.bf16_bits_to_f32(np.frombuffer(blob, np.uint16, count=c0 * 32, offset=woff)).reshape(c0, 32)[:, :27]
-            w = w.reshape(c0, 3, 3, 3).transpose(0, 3, 1, 2)
-            bias = np.frombuffer(blob, np.float32, count=c0, offset=boff)
-            ref = onet.silu(onet.conv2d(x, np.ascontiguousarray(w), bias, 2, 1))
-            got = buf(ob)[..., ooff:ooff + c0].transpose(0, 3, 1, 2)
-            assert _rel_l2(got, ref) < 4e-3
-        elif op[0] == eng_mod.OP_POOL:
-            _, b_, off, c = op[:4]
-            y = buf(b_)[..., off:off + c].transpose(0, 3, 1, 2)
-            for j in range(1, 4):
-                y = onet.maxpool5(y)
-                np.testing.assert_array_equal(buf(b_)[..., off + j * c:off + (j + 1) * c].transpose(0, 3, 1, 2), y)
-        elif op[0] == eng_mod.OP_UP:
-            _, ib, ioff, c, scale, ob, ooff = op[:7]
-            src = buf(ib)[..., ioff:ioff + c]
-            ref = src.repeat(scale, axis=1).repeat(scale, axis=2)
-            np.testing.assert_array_equal(buf(ob)[..., ooff:ooff + c], ref)
-    _diag(f"per-layer parity {name} {B}x{H}x{W}: {len(P.ops)} launches, worst conv rel-L2 {worst:.2e}")
+    rep = []
+    worst = plan_ref.check_plan(eng, xt, report=rep)
+    kinds = sorted({k for _, k, _ in rep})
+    assert ("dfl" in kinds and "cls" in kinds) == (head != "unfused"), kinds
+    _diag(f"per-layer parity {name} {B}x{H}x{W} {head}: {len(eng.plan.ops)} launches ({', '.join(kinds)}), worst conv rel-L2 {worst:.2e}")
+    eng.close()
 
 
 def test_engine_graph_and_end_to_end_drift(n_p2):

@@ -41,6 +41,10 @@ CONV_CASES = [
     (1, 40, 40, 16, 32, 3, 1, True, True),
     (1, 64, 64, 192, 96, 1, 1, True, False),      # K = 3 chunks of 64
     (4, 5, 7, 160, 160, 3, 1, True, False),       # x-scale widths, tiny maps, several images per tile
+    # more tiles than the 2 x 148 CTA slots: every CTA runs several tiles (accumulator ring, alternate MMA warps, bias reload)
+    (4, 128, 160, 32, 32, 3, 1, True, False),     # 3x3 stride 1, 81920 output pixels
+    (3, 256, 320, 32, 64, 3, 2, True, False),     # stride 2, 61440 output pixels
+    (4, 64, 96, 64, 512, 1, 1, True, False),      # Cout 512: two N tiles per pixel tile, 24576 pixels
 ]
 
 
@@ -66,6 +70,7 @@ CHAIN_CASES = [
     (3, 16, 24, 16, 16, 1, True, 32, 32, True),          # yolov8n widths: 32-byte rows, extra source of 32
     (1, 130, 70, 32, 64, 2, False, 0, 64, True),         # stride 2, ragged 65 x 35 output, many tiles per CTA
     (2, 24, 24, 48, 48, 1, True, 96, 96, True),          # K blocks 64 + 32 (extra) and 32 + 16 (main)
+    (4, 256, 320, 32, 64, 2, False, 0, 64, True),        # 81920 output pixels: the look-ahead loads and double buffers of many tiles per CTA
 ]
 
 
@@ -166,7 +171,10 @@ def test_conv_channel_slices_and_strides():
     assert np.all(got[..., :64] == 7.0) and np.all(got[..., 96:] == 7.0)      # neighbours untouched
 
 
-@pytest.mark.parametrize("shape", [(2, 16, 24, 64, 32, 48), (1, 32, 40, 128, 64, 96), (3, 8, 8, 32, 80, 64), (1, 6, 10, 256, 128, 128)])
+UPCAT_CASES = [(2, 16, 24, 64, 32, 48), (1, 32, 40, 128, 64, 96), (3, 8, 8, 32, 80, 64), (1, 6, 10, 256, 128, 128)]     # B, H, W, C0, C1, Cout
+
+
+@pytest.mark.parametrize("shape", UPCAT_CASES)
 def test_conv_over_upsample_concat_matches_oracle(shape):
     """C2f.cv1 over Concat([Upsample(x_lo), skip]) (yolov8-p2.yaml:33-36) with the upsample and the concat folded
     into the conv's TMA loads (zero-stride tensor-map dimensions replicate each low-resolution pixel 2x2)."""
@@ -207,19 +215,35 @@ def test_conv_rejects_bad_arguments():
         ops.conv2d_bf16(x, w, torch.zeros(16, device="cuda"), 5)            # k = 5 unsupported
 
 
-@pytest.mark.parametrize("hw,src,pad", [((64, 96), (64, 96), (0, 0)), ((64, 96), (52, 96), (6, 0)), ((32, 64), (32, 50), (0, 7))])
-def test_stem_u8_matches_oracle(hw, src, pad):
+STEM_CASES = [
+    # B, canvas, frame, (pad top, pad left), C0
+    (2, (64, 96), (64, 96), (0, 0), 16),
+    (2, (64, 96), (52, 96), (6, 0), 16),
+    (2, (32, 64), (32, 50), (0, 7), 16),
+    # several tiles per CTA (16 x 8 output pixels per tile, up to 8 CTAs per SM): the next-patch prefetch and the mixed-radix
+    # tile advance with the grid stride above the tiles per image (160) ...
+    (16, (256, 320), (256, 320), (0, 0), 16),
+    (16, (256, 320), (256, 320), (0, 0), 32),
+    # ... and below them (3200 tiles per image)
+    (1, (1280, 1280), (1280, 1280), (0, 0), 32),
+    # many small padded images (12 tiles per image), the x-scale stem width
+    (128, (64, 96), (52, 96), (6, 0), 80),
+    (128, (64, 96), (64, 90), (0, 3), 32),
+]
+
+
+@pytest.mark.parametrize("B,hw,src,pad,C0", STEM_CASES, ids=[f"hw{i}-src{i}-pad{i}" for i in range(len(STEM_CASES))])
+def test_stem_u8_matches_oracle(B, hw, src, pad, C0):
     """Letterbox pad (114) + BGR->RGB + /255 + Conv(3->C0, k3, s2) + SiLU on raw uint8 frames."""
     from b200dt import ops
 
     torch = _t()
     g = np.random.default_rng(2)
     H, W = hw
-    frames = g.integers(0, 256, (2, src[0], src[1], 3), dtype=np.uint8)
-    C0 = 16
+    frames = g.integers(0, 256, (B, src[0], src[1], 3), dtype=np.uint8)
     w = (g.standard_normal((C0, 3, 3, 3)) / 3.0).astype(np.float32)
     b = (0.1 * g.standard_normal(C0)).astype(np.float32)
-    canvas = np.full((2, H, W, 3), 114, np.uint8)
+    canvas = np.full((B, H, W, 3), 114, np.uint8)
     canvas[:, pad[0]:pad[0] + src[0], pad[1]:pad[1] + src[1]] = frames
     x = pp.preprocess(list(canvas))
     ref = onet.bf16_round(onet.silu(onet.conv2d(x, onet.bf16_round(w), b, 2, 1)))     # bf16 weights, exact uint8 inputs
