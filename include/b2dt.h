@@ -210,6 +210,9 @@ int b2_tracker_create_ex(int n_streams, int capacity, int max_dets, int max_lost
                          float iou_threshold, int mode, b2_tracker_t** out);
 int b2_tracker_destroy(b2_tracker_t* t);
 int b2_tracker_reset(b2_tracker_t* t, void* stream);
+/* b2_tracker_reset for the streams with flags_dev[s] != 0 ([n_streams] int32, device): their slots, counters, frame count and
+ * mode-1 fields are cleared and next_id set to 1; other streams are not touched.  Ordered on `stream`, no host synchronisation. */
+int b2_tracker_reset_streams(b2_tracker_t* t, const int32_t* flags_dev, void* stream);
 /* The reference's track list is unbounded (enhanced_multi_target_tracker.py:92-101 appends); the bank is not.  A caller that
  * sees `active + max_dets > capacity` (b2_tracker_stats / b2_tracker_export) enlarges the bank in place: every slot keeps its
  * index, state and id.  Synchronises `stream`.  Output buffers of b2_tracker_update must be re-sized by the caller. */
@@ -311,6 +314,53 @@ int b2_reid_gather(const void* const* level_ptr, const int* level_h, const int* 
  * smooth = 0.9 smooth + 0.1 curr, otherwise smooth = curr; then smooth /= |smooth| (a first smooth is the same vector as curr in
  * the reference, so curr receives that renormalisation too). */
 int b2_reid_update(float* curr, float* smooth, const uint8_t* has_smooth, int N, int D, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Global camera motion (camera_motion_compensation/global_motion_detector.py, method 'optical_flow', and the global-reset rule of
+ * motion_compensated_multi_tracker.py:75-146), batched over S streams.  Frames are HWC BGR uint8 at per-stream byte offsets
+ * (frame_off_dev, int64 [S], the layout of b2_letterbox_u8).  Only the reference's parameters are supported; others return
+ * B2_ERR_UNSUPPORTED.  Frames of any size: LK starts, per stream, at the deepest level larger than the 21x21 window (cv2's rule).
+ * ---------------------------------------------------------------------------------------------- */
+/* Host-only layout of a gray pyramid buffer (4 levels per stream, back to back): shapes_host [S][2] {h, w};
+ * level_off_host [S][4] byte offsets, level_hw_host [S][4][2], pix_off_host [S] offsets of level 0 in pixels (the response buffer
+ * of b2_corner_min_eig), totals_host [2] {pyramid bytes, level-0 pixels}. */
+int b2_pyramid_layout(int n_streams, const int* shapes_host, long long* level_off_host, int* level_hw_host, long long* pix_off_host,
+                      long long* totals_host);
+/* cv2.cvtColor(BGR2GRAY) and three cv2.pyrDown levels, bit-exact.  max_h / max_w: the largest frame. */
+int b2_gray_pyramid_u8(const uint8_t* frames, const long long* frame_off_dev, int n_streams, int max_h, int max_w,
+                       uint8_t* pyr, const long long* level_off_dev, const int* level_hw_dev, void* stream);
+/* cv2.cornerMinEigenVal(level 0, blockSize=7, ksize=3) -> eig_out fp32 at pix_off (within 1e-5 of the maximum of cv2's). */
+int b2_corner_min_eig(const uint8_t* pyr, const long long* level_off_dev, const int* level_hw_dev, const long long* pix_off_dev,
+                      int n_streams, int max_h, int max_w, int block_size, int ksize, float* eig_out, void* stream);
+/* goodFeaturesToTrack's selection (maxCorners=200, qualityLevel=0.01, minDistance=15) on a response: local 3x3 maxima above
+ * 0.01 max off the one-pixel border, ordered by value then linear index (both descending), accepted greedily at squared distance
+ * >= 225.  corners_out [S][200][2] fp32 (x, y), counts_out [S].  workspace: b2_good_features_workspace_bytes(S, total_pixels). */
+size_t b2_good_features_workspace_bytes(int n_streams, long long total_pixels);
+int b2_good_features(const float* eig, const long long* pix_off_dev, const int* level_hw_dev, int n_streams, int max_h, int max_w,
+                     long long total_pixels, int max_corners, double quality_level, double min_distance, void* workspace,
+                     size_t workspace_bytes, float* corners_out, int* counts_out, void* stream);
+/* cv2.calcOpticalFlowPyrLK(winSize=21x21, maxLevel=3, criteria COUNT|EPS 30 / 0.01) between two pyramids of the same layout:
+ * pts [S][max_pts][2], counts [S]; next_out [S][max_pts][2], status_out [S][max_pts] uint8 (rows past a count are not written). */
+int b2_lk_pyr(const uint8_t* prev_pyr, const uint8_t* next_pyr, const long long* level_off_dev, const int* level_hw_dev, int n_streams,
+              const float* pts, const int* counts, int max_pts, int win, int max_level, int max_count, double epsilon,
+              float* next_out, uint8_t* status_out, void* stream);
+
+/* The per-stream detector and its decision state on the device.  b2_motion_flow: pyramid of the frame (the previous frame's is
+ * kept), then corners of the previous frame and their flow into this one -- needs the frames only.  b2_motion_decide (once per
+ * flow): detect_motion's vector / thresholds and _should_global_reset from det_counts_dev [S] (this frame's detections, NULL = 0);
+ * flags_dev [S] int32 = 1 where every track of the stream is to be dropped (feed b2_tracker_reset_streams); info_dev [S][8] fp32
+ * {magnitude, vx, vy, is_motion, should_reset, global_reset, corners, tracked}.  tracker_stats_dev (b2_tracker_stats of the bank
+ * before the reset, may be NULL) feeds the individual-resets / recoveries base.  b2_motion_stats: [S][8] float64 {total_detections,
+ * motion_events, reset_triggers, avg_motion_magnitude, global_motion_events, global_resets, base individual_resets,
+ * base tracking_recoveries}. */
+typedef struct b2_motion b2_motion_t;
+int b2_motion_create(int n_streams, const int* shapes_host, b2_motion_t** out);
+int b2_motion_flow(b2_motion_t* m, const uint8_t* frames, const long long* frame_off_dev, void* stream);
+int b2_motion_decide(b2_motion_t* m, const int32_t* det_counts_dev, const long long* tracker_stats_dev, int32_t* flags_dev,
+                     float* info_dev, void* stream);
+int b2_motion_stats(b2_motion_t* m, double* stats_dev_out, void* stream);
+int b2_motion_reset(b2_motion_t* m, void* stream);
+int b2_motion_destroy(b2_motion_t* m);
 
 #ifdef __cplusplus
 }

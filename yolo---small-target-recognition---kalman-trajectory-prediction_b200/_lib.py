@@ -58,6 +58,7 @@ SIGNATURES = {
     "b2_tracker_create_ex": (c_int, [c_int, c_int, c_int, c_int, c_int, c_float, c_int, C.POINTER(_P)]),
     "b2_tracker_destroy": (c_int, [_P]),
     "b2_tracker_reset": (c_int, [_P, _P]),
+    "b2_tracker_reset_streams": (c_int, [_P, _P, _P]),
     "b2_tracker_capacity": (c_int, [_P]),
     "b2_tracker_grow": (c_int, [_P, c_int, _P]),
     "b2_tracker_stats": (c_int, [_P, _P, _P]),
@@ -80,6 +81,18 @@ SIGNATURES = {
     "b2_botsort_cost": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, C.c_double, _P, _P]),
     "b2_reid_gather": (c_int, [_P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_int, _P, _P]),
     "b2_reid_update": (c_int, [_P, _P, _P, c_int, c_int, _P]),
+    "b2_pyramid_layout": (c_int, [c_int, _P, _P, _P, _P, _P]),
+    "b2_gray_pyramid_u8": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P, _P, _P]),
+    "b2_corner_min_eig": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    "b2_good_features_workspace_bytes": (c_size_t, [c_int, C.c_longlong]),
+    "b2_good_features": (c_int, [_P, _P, _P, c_int, c_int, c_int, C.c_longlong, c_int, C.c_double, C.c_double, _P, c_size_t, _P, _P, _P]),
+    "b2_lk_pyr": (c_int, [_P, _P, _P, _P, c_int, _P, _P, c_int, c_int, c_int, c_int, C.c_double, _P, _P, _P]),
+    "b2_motion_create": (c_int, [c_int, _P, C.POINTER(_P)]),
+    "b2_motion_flow": (c_int, [_P, _P, _P, _P]),
+    "b2_motion_decide": (c_int, [_P, _P, _P, _P, _P, _P]),
+    "b2_motion_stats": (c_int, [_P, _P, _P]),
+    "b2_motion_reset": (c_int, [_P, _P]),
+    "b2_motion_destroy": (c_int, [_P]),
 }
 
 B2_OK, B2_ERR_ARG, B2_ERR_CUDA, B2_ERR_STATE, B2_ERR_UNSUPPORTED = 0, -1, -2, -3, -4

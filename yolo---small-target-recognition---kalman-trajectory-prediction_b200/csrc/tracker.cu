@@ -28,6 +28,7 @@
 // order.  List order of the reference (= ascending track id) is carried by the id column; slots are recycled.
 #include "common.cuh"
 
+#include <algorithm>
 #include <new>
 
 void b2_count_launch(int n);
@@ -1176,6 +1177,60 @@ __global__ void regrid_kernel(const uint32_t* __restrict__ src, uint32_t* __rest
 }
 __global__ void fill_i32(int32_t* p, int n, int v) { const int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = v; }
 
+// b2_tracker_reset_streams: every word a flagged stream owns in the arena -- its slots of each [field][N] plane, its candidate
+// lists, sweep scratch and pairs, counters and stats -- set to what b2_tracker_reset leaves (0, next_id = 1).
+__device__ __forceinline__ uint32_t* stream_word(const Bank& b, int s, long long i) {
+    const int n_planes = NFF + NIF + 2 * kVelRing + 2 * kTraj + (b.mode ? MR_NF + MR_NI : 0) + 3;
+    const long long C = b.C, N = b.N;
+    if (i < n_planes * C) {
+        int q = (int)(i / C);
+        const long long g = (long long)s * C + i % C;
+        if (q < NFF) return (uint32_t*)b.f + q * N + g;
+        q -= NFF;
+        if (q < NIF) return (uint32_t*)b.i + q * N + g;
+        q -= NIF;
+        if (q < 2 * kVelRing) return (uint32_t*)b.vel + q * N + g;
+        q -= 2 * kVelRing;
+        if (q < 2 * kTraj) return (uint32_t*)b.traj + q * N + g;
+        q -= 2 * kTraj;
+        if (b.mode) {
+            if (q < MR_NF) return (uint32_t*)b.mrf + q * N + g;
+            q -= MR_NF;
+            if (q < MR_NI) return (uint32_t*)b.mri + q * N + g;
+            q -= MR_NI;
+        }
+        return (uint32_t*)(q == 0 ? b.ctrk_slot : q == 1 ? b.cid : b.cmatch) + g;
+    }
+    i -= n_planes * C;
+    if (i < 4 * C) return (uint32_t*)b.cbox + 4 * C * s + i;
+    i -= 4 * C;
+    if (i < 4ll * b.pair_cap) return (uint32_t*)b.pairs + 4ll * b.pair_cap * s + i;
+    i -= 4ll * b.pair_cap;
+    if (i < 2ll * b.nchunks) return (uint32_t*)b.agg + 2ll * b.nchunks * s + i;
+    i -= 2ll * b.nchunks;
+    if (i < b.nchunks) return (uint32_t*)b.chunk_free + (long long)b.nchunks * s + i;
+    i -= b.nchunks;
+    if (i < 4) return (uint32_t*)b.fcnt + 4 * s + i;
+    i -= 4;
+    if (i < 16) return (uint32_t*)b.stats + 16 * s + i;
+    i -= 16;
+    return i == 0 ? (uint32_t*)b.frame_count + s : i == 1 ? (uint32_t*)b.next_id + s : nullptr;
+}
+
+long long stream_words(const Bank& b) {
+    const int n_planes = NFF + NIF + 2 * kVelRing + 2 * kTraj + (b.mode ? MR_NF + MR_NI : 0) + 3;
+    return (long long)(n_planes + 4) * b.C + 4ll * b.pair_cap + 3ll * b.nchunks + 4 + 16 + 2;
+}
+
+__global__ void __launch_bounds__(256) reset_streams_kernel(const Bank b, const int32_t* __restrict__ flags, long long n_words) {
+    const int s = blockIdx.y;
+    if (!flags[s]) return;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_words; i += (long long)gridDim.x * blockDim.x) {
+        uint32_t* w = stream_word(b, s, i);
+        *w = i == n_words - 1 ? 1u : 0u;     // the last word is next_id
+    }
+}
+
 struct Layout { size_t f, i, v, t, rf, ri, agg, cf, fc, tk, cs, cb, ci, cm, pr, ni, fcn, st, total; };
 
 Layout bank_layout(int S, int C, int max_dets, int nchunks, int pair_cap, int mode) {
@@ -1259,6 +1314,17 @@ extern "C" int b2_tracker_reset(b2_tracker_t* t, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
     B2_CUDA(cudaMemsetAsync(t->impl.arena, 0, t->impl.arena_bytes, st));
     fill_i32<<<b2_ceil_div(t->impl.b.S, 256), 256, 0, st>>>(t->impl.b.next_id, t->impl.b.S, 1);   // next_track_id = 1 (:30)
+    B2_CUDA(cudaGetLastError());
+    b2_count_launch(1);
+    return B2_OK;
+}
+
+extern "C" int b2_tracker_reset_streams(b2_tracker_t* t, const int32_t* flags_dev, void* stream) {
+    B2_REQUIRE(t && flags_dev, "tracker_reset_streams: null argument");
+    const Bank& b = t->impl.b;
+    const long long n = stream_words(b);
+    const int blocks = (int)std::min<long long>(b2_ceil_div((int)std::min<long long>(n, 1ll << 30), 256), 64);
+    reset_streams_kernel<<<dim3(blocks, b.S), 256, 0, (cudaStream_t)stream>>>(b, flags_dev, n);
     B2_CUDA(cudaGetLastError());
     b2_count_launch(1);
     return B2_OK;

@@ -6,6 +6,10 @@
   decode                 Detect._inference (ultralytics/nn/modules/head.py:152-187) + candidate filter
   nms                    tail of non_max_suppression (ultralytics/utils/nms.py:129-160) + scale_boxes
   non_max_suppression    the reference signature (ultralytics/utils/nms.py:13-167) on a (B, 4+nc, A) tensor
+  gray_pyramid_u8        cv2.cvtColor(BGR2GRAY) + three cv2.pyrDown levels of S frames (bit-exact), as a :class:`GrayPyramid`
+  corner_min_eig         cv2.cornerMinEigenVal(gray, 7, 3)
+  good_features_to_track cv2.goodFeaturesToTrack(maxCorners=200, qualityLevel=0.01, minDistance=15, blockSize=7) per stream
+  optical_flow_pyr_lk    cv2.calcOpticalFlowPyrLK(winSize=(21, 21), maxLevel=3, criteria=(COUNT|EPS, 30, 0.01)) per stream
 
 Every function needs a CUDA device and raises if the library is missing: there is no CPU fallback.
 torch is used for device memory and streams only.
@@ -167,6 +171,119 @@ def letterbox_u8(packed, offsets, geom, H, W, out=None, stream=None):
     assert offsets.dtype == torch.int64 and geom.dtype == torch.int32 and offsets.shape[0] == B and tuple(geom.shape) == (B, 6)
     _lib.check(lib.b2_letterbox_u8(_lib.ptr(packed), _lib.ptr(offsets), _lib.ptr(geom), B, H, W, _lib.ptr(out), _lib.stream_ptr(stream)))
     return out
+
+
+def pyramid_layout(shapes):
+    """Layout of the gray pyramids of frames of ``shapes`` [(h, w), ...] (host only): level byte offsets int64 [S][4], level shapes
+    int32 [S][4][2], level-0 pixel offsets int64 [S], total bytes, total level-0 pixels."""
+    lib = _lib.load()
+    S = len(shapes)
+    sh = np.ascontiguousarray(np.asarray(shapes, np.int32).reshape(S, 2))
+    off, hw, pix, tot = np.zeros((S, 4), np.int64), np.zeros((S, 4, 2), np.int32), np.zeros((S,), np.int64), np.zeros((2,), np.int64)
+    _lib.check(lib.b2_pyramid_layout(S, sh.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.c_void_p), hw.ctypes.data_as(C.c_void_p),
+                                     pix.ctypes.data_as(C.c_void_p), tot.ctypes.data_as(C.c_void_p)))
+    return off, hw, pix, int(tot[0]), int(tot[1])
+
+
+class GrayPyramid:
+    """The 4-level gray pyramids of S frames in one CUDA uint8 buffer (``pyramid_layout``); ``level(s, l)`` is a [h][w] view."""
+
+    def __init__(self, shapes, device=None):
+        torch = _torch()
+        dev = device or _lib.require_cuda()
+        self.shapes = [(int(h), int(w)) for h, w in shapes]
+        self.S = len(self.shapes)
+        self.level_off, self.level_hw, self.pix_off, nbytes, self.npix = pyramid_layout(self.shapes)
+        self.max_h, self.max_w = max(h for h, _ in self.shapes), max(w for _, w in self.shapes)
+        self.buf = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+        self.off_dev, self.hw_dev, self.pix_dev = (torch.from_numpy(a).to(dev) for a in (self.level_off, self.level_hw, self.pix_off))
+
+    def level(self, s, l):
+        h, w = (int(v) for v in self.level_hw[s, l])
+        o = int(self.level_off[s, l])
+        return self.buf[o:o + h * w].view(h, w)
+
+    def plane(self, flat, s):
+        """Stream ``s``'s [h][w] view of a level-0-sized per-pixel buffer (``corner_min_eig``)."""
+        h, w = self.shapes[s]
+        o = int(self.pix_off[s])
+        return flat[o:o + h * w].view(h, w)
+
+
+def frame_offsets(frames, shapes):
+    """Byte offsets (int64 numpy [S]) of the frames in ``frames``: a CUDA uint8 [S][h][w][3] batch, or the 1-D ``pack_frames`` layout."""
+    if frames.dim() == 4:
+        S, h, w, _ = frames.shape
+        return np.arange(S, dtype=np.int64) * (h * w * 3)
+    offs, n = pack_layout(shapes)
+    if frames.numel() != n:
+        raise ValueError(f"packed frames: expected {n} bytes for shapes {shapes}, got {frames.numel()}")
+    return offs
+
+
+def gray_pyramid_u8(frames, shapes=None, out=None, stream=None):
+    """cv2.cvtColor(COLOR_BGR2GRAY) + three cv2.pyrDown levels of S HWC BGR uint8 frames, bit-exact.  frames: CUDA uint8
+    [S][h][w][3], or 1-D packed by ``pack_frames`` with their ``shapes``.  Returns (or fills) a :class:`GrayPyramid`."""
+    torch = _torch()
+    lib = _lib.load()
+    assert frames.is_cuda and frames.dtype == torch.uint8 and frames.is_contiguous()
+    if shapes is None:
+        shapes = [tuple(frames.shape[1:3])] * frames.shape[0]
+    pyr = out or GrayPyramid(shapes, frames.device)
+    offs = torch.from_numpy(frame_offsets(frames, shapes)).to(frames.device)
+    _lib.check(lib.b2_gray_pyramid_u8(_lib.ptr(frames), _lib.ptr(offs), pyr.S, pyr.max_h, pyr.max_w, _lib.ptr(pyr.buf), _lib.ptr(pyr.off_dev),
+                                      _lib.ptr(pyr.hw_dev), _lib.stream_ptr(stream)))
+    return pyr
+
+
+def corner_min_eig(pyr, block_size=7, ksize=3, stream=None):
+    """cv2.cornerMinEigenVal(level 0, blockSize, ksize) of every stream of a :class:`GrayPyramid`: float32 CUDA [npix]
+    (``pyr.plane(out, s)`` is stream s).  Only blockSize=7, ksize=3 (the reference's) are provided."""
+    torch = _torch()
+    out = torch.empty((pyr.npix,), dtype=torch.float32, device=pyr.buf.device)
+    _lib.check(_lib.load().b2_corner_min_eig(_lib.ptr(pyr.buf), _lib.ptr(pyr.off_dev), _lib.ptr(pyr.hw_dev), _lib.ptr(pyr.pix_dev), pyr.S,
+                                             pyr.max_h, pyr.max_w, int(block_size), int(ksize), _lib.ptr(out), _lib.stream_ptr(stream)))
+    return out
+
+
+def good_features_to_track(pyr, max_corners=200, quality_level=0.01, min_distance=15, block_size=7, eig=None, stream=None):
+    """cv2.goodFeaturesToTrack(level 0, maxCorners, qualityLevel, minDistance, blockSize=blockSize) for every stream of a
+    :class:`GrayPyramid`; ``eig`` (``corner_min_eig``'s output) is computed when None.  Returns (corners float32 CUDA
+    [S][200][2] (x, y), counts int32 CUDA [S]); rows past a stream's count are not written."""
+    torch = _torch()
+    lib = _lib.load()
+    if eig is None:
+        eig = corner_min_eig(pyr, block_size, 3, stream)
+    elif block_size != 7:
+        raise NotImplementedError("good_features_to_track: only blockSize=7")
+    dev = pyr.buf.device
+    wsb = lib.b2_good_features_workspace_bytes(pyr.S, pyr.npix)
+    ws = torch.empty((wsb,), dtype=torch.uint8, device=dev)
+    corners = torch.zeros((pyr.S, int(max_corners), 2), dtype=torch.float32, device=dev)
+    counts = torch.zeros((pyr.S,), dtype=torch.int32, device=dev)
+    _lib.check(lib.b2_good_features(_lib.ptr(eig), _lib.ptr(pyr.pix_dev), _lib.ptr(pyr.hw_dev), pyr.S, pyr.max_h, pyr.max_w, pyr.npix,
+                                    int(max_corners), float(quality_level), float(min_distance), _lib.ptr(ws), wsb, _lib.ptr(corners),
+                                    _lib.ptr(counts), _lib.stream_ptr(stream)))
+    return corners, counts
+
+
+def optical_flow_pyr_lk(prev, nxt, pts, counts=None, win_size=(21, 21), max_level=3, criteria=(3, 30, 0.01), stream=None):
+    """cv2.calcOpticalFlowPyrLK(prev, next, pts, None, winSize, maxLevel, criteria) per stream between two :class:`GrayPyramid`
+    of the same shapes.  pts: CUDA float32 [S][P][2]; counts: CUDA int32 [S] (None: P each).  Returns (next points float32
+    [S][P][2], status uint8 [S][P]); rows past a count are not written.  criteria must include COUNT and EPS (type 3)."""
+    torch = _torch()
+    assert prev.shapes == nxt.shapes and pts.is_cuda and pts.dtype == torch.float32 and pts.is_contiguous() and pts.shape[0] == prev.S
+    if int(criteria[0]) != 3 or tuple(win_size) != (21, 21):
+        raise NotImplementedError("optical_flow_pyr_lk: only winSize=(21, 21), criteria type COUNT|EPS")
+    P = pts.shape[1]
+    if counts is None:
+        counts = torch.full((prev.S,), P, dtype=torch.int32, device=pts.device)
+    out = torch.zeros_like(pts)
+    status = torch.zeros((prev.S, P), dtype=torch.uint8, device=pts.device)
+    _lib.check(_lib.load().b2_lk_pyr(_lib.ptr(prev.buf), _lib.ptr(nxt.buf), _lib.ptr(prev.off_dev), _lib.ptr(prev.hw_dev), prev.S,
+                                     _lib.ptr(pts), _lib.ptr(counts), P, int(win_size[0]), int(max_level), int(criteria[1]),
+                                     float(criteria[2]), _lib.ptr(out), _lib.ptr(status), _lib.stream_ptr(stream)))
+    return out, status
 
 
 def sppf_pool(buf, coff, c, stream=None):

@@ -15,7 +15,7 @@ from __future__ import annotations
 
 from . import _lib, cfg, ops, weights
 from .predictor import DetectPipeline, letterbox_table
-from .tracker import TrackerBank
+from .tracker import GlobalMotionBank, TrackerBank
 
 
 def bind_host_to_gpu(gpu_index):
@@ -50,7 +50,7 @@ def shard_streams(n_streams, rank, world_size):
 class DetectTrackPipeline:
     def __init__(self, model="yolov8s-p2", n_streams=1, frame_hw=(512, 640), imgsz=640, conf=0.15, iou=0.6, max_det=300,
                  max_lost_frames=150, min_hits=1, iou_threshold=0.1, capacity=512, state_dict=None, seed=0, nc=None,
-                 nms_mode="exact", overlap_post=False, max_tracks_out=None):
+                 nms_mode="exact", overlap_post=False, max_tracks_out=None, tracker="enhanced"):
         """overlap_post: run NMS + tracker of step t on a second CUDA stream while the forward of step t+1 runs on the
         caller's stream (the small latency-bound launches fill the tails of the conv kernels).  The returned device
         tensors are then valid only after ``join()``.
@@ -62,8 +62,16 @@ class DetectTrackPipeline:
         all share one shape needing no resize take the frames as [S][h][w][3] and letterbox inside the stem kernel.  Any other
         set of shapes (mixed, or one shape that needs a resize) is the general path: frames are packed back to back
         (``ops.pack_frames``), letterboxed on the GPU into one canvas -- ``auto`` padding for one common shape, the full imgsz
-        canvas for mixed shapes, as YOLO.predict does -- and NMS scales each stream's boxes to its own frame."""
+        canvas for mixed shapes, as YOLO.predict does -- and NMS scales each stream's boxes to its own frame.
+        tracker: "enhanced" (EnhancedMultiTargetTracker per stream) or "motion_compensated" (MotionCompensatedMultiTracker per
+        stream, ``update(dets, frame)``): a mode-1 bank, and the camera-motion detector on the GPU (:class:`GlobalMotionBank`) --
+        its flow on the uploaded frames, its decision after NMS, and a reset of the streams it flags before the tracker update.
+        ``results()`` then also fills ``host_extra`` [S][max_tracks_out][4] (reset_count, frames_since_reset as int32 bits,
+        motion_consistency) and ``host_motion`` [S][8] (``GlobalMotionBank.decide``'s info)."""
         import torch
+
+        if tracker not in ("enhanced", "motion_compensated"):
+            raise ValueError(f"tracker={tracker!r}: 'enhanced' or 'motion_compensated'")
 
         self.device = _lib.require_cuda()
         self.spec = cfg.resolve(model, nc=nc)
@@ -82,8 +90,13 @@ class DetectTrackPipeline:
         self.conf, self.iou, self.nms_mode = float(conf), float(iou), nms_mode
         self.detect = DetectPipeline(self.spec, sd, self.S, self.H, self.W, max_det)
         self.max_det = int(max_det)
+        self.tracker = tracker
         self.bank = TrackerBank(self.S, capacity, max_det, max_lost_frames, min_hits, iou_threshold,
-                                max_out=min(int(max_tracks_out), int(capacity)) if max_tracks_out else None)
+                                max_out=min(int(max_tracks_out), int(capacity)) if max_tracks_out else None,
+                                mode=1 if tracker == "motion_compensated" else 0)
+        self.motion = GlobalMotionBank(self.S, self.frame_shapes, self.device) if tracker == "motion_compensated" else None
+        if self.motion is not None:
+            self._tstats = torch.zeros((self.S, 8), dtype=torch.int64, device=self.device)
         self._fixed_out = bool(max_tracks_out)
         self.flops_per_frame = self.detect.engine.flops_per_image
         # double-buffered staging for the host-facing path
@@ -108,6 +121,7 @@ class DetectTrackPipeline:
         self._rows_downloaded = torch.cuda.Event()
         self._rows_downloaded.record()
         self.h2d_bytes_per_step = self._dev_frames[0].numel()
+        self._regrow_host = False
         self._alloc_host()
 
     def _alloc_host(self):
@@ -117,6 +131,11 @@ class DetectTrackPipeline:
         self.host_counts = torch.zeros((self.S,), dtype=torch.int32).pin_memory()
         self.host_stats = torch.zeros((self.S, 8), dtype=torch.int64).pin_memory()
         self.d2h_bytes_per_step = self.host_rows.numel() * 4 + self.host_counts.numel() * 4 + self.host_stats.numel() * 8
+        self.host_extra = self.host_motion = None
+        if self.motion is not None:
+            self.host_extra = torch.empty((self.S, self.bank.max_out, 4), dtype=torch.float32).pin_memory()
+            self.host_motion = torch.empty((self.S, 8), dtype=torch.float32).pin_memory()
+            self.d2h_bytes_per_step += self.host_extra.numel() * 4 + self.host_motion.numel() * 4
 
     def _packed(self, frames):
         """The general path's input: ``packed_bytes`` uint8 in the ``ops.pack_frames`` layout (any shape with that many bytes,
@@ -126,6 +145,15 @@ class DetectTrackPipeline:
                              f"got {frames.dtype} {tuple(frames.shape)}")
         return frames.view(-1)
 
+    def _motion_flow(self, frames_u8, stream):
+        self.motion.flow(frames_u8, self._offsets if self.ragged else None, stream)
+
+    def _motion_reset(self, counts, stream):
+        """The decision after NMS and the reset of the flagged streams (MotionCompensatedMultiTracker.update :279-293)."""
+        self.bank.stats_async(stream, out=self._tstats)
+        flags, _ = self.motion.decide(counts, self._tstats, stream)
+        self.bank.reset_streams(flags, stream)
+
     def step_device(self, frames_u8, with_trajectory=False, stream=None):
         """frames_u8: CUDA uint8 [S][h][w][3] BGR, or on the general path (mixed / resized shapes) the packed frames of
         ``ops.pack_frames``.  Returns (track rows [S][capacity][20], counts [S]) on the GPU."""
@@ -133,6 +161,8 @@ class DetectTrackPipeline:
 
         cur = stream or torch.cuda.current_stream()
         if not self.overlap_post:
+            if self.motion is not None:
+                self._motion_flow(frames_u8, stream)
             if self.ragged:
                 dets, counts = self.detect.run_ragged(self._packed(frames_u8), self._offsets, self._geom, self._scale, self.conf, self.iou,
                                                       None, False, self.nms_mode, stream)
@@ -141,8 +171,11 @@ class DetectTrackPipeline:
                                            self.nms_mode, stream)
             # the bank's row block is about to be rewritten: a download of the previous step's rows (step_host) must be over
             cur.wait_event(self._rows_downloaded)
+            if self.motion is not None:
+                self._motion_reset(counts, stream)
             return self.bank.update(dets, counts, with_trajectory=with_trajectory, stream=stream)
         d, ps = self.detect, self._post_stream
+        frames_in = frames_u8
         if self.ragged:
             frames_u8 = d.letterbox(self._packed(frames_u8), self._offsets, self._geom, stream)
         if self.forward_events is not None:           # bench.py: CUDA events around the forward graph, on the stream it runs on
@@ -154,6 +187,8 @@ class DetectTrackPipeline:
             ev[1].record(cur)
             self.forward_events.append(ev)
         cur.wait_event(self._post_done)               # NMS of the previous step has read the candidate lists
+        if self.motion is not None:                   # ... and its motion decision has read the flow of the previous frame
+            self._motion_flow(frames_in, stream)
         d.candidates(self.conf, None, stream)
         self._cand_done.record(cur)
         ps.wait_event(self._cand_done)
@@ -162,6 +197,8 @@ class DetectTrackPipeline:
             dets, counts = d.nms(self.iou, None, False, self.nms_mode, ps, self._scale)
         else:
             dets, counts = d.nms(self.iou, (self.h0, self.w0), False, self.nms_mode, ps)
+        if self.motion is not None:
+            self._motion_reset(counts, ps)
         out = self.bank.update(dets, counts, with_trajectory=with_trajectory, stream=ps)
         self._post_done.record(ps)
         return out
@@ -173,6 +210,9 @@ class DetectTrackPipeline:
         import torch
 
         cur = torch.cuda.current_stream()
+        if self._regrow_host:
+            self._alloc_host()
+            self._regrow_host = False
         k = self._slot
         self._slot ^= 1
         with torch.cuda.stream(self._copy_stream):
@@ -192,6 +232,9 @@ class DetectTrackPipeline:
             self.host_rows.copy_(rows, non_blocking=True)
             self.host_counts.copy_(counts, non_blocking=True)
             self.host_stats.copy_(self.bank.stats_async(self._d2h_stream), non_blocking=True)
+            if self.motion is not None:
+                self.host_extra.copy_(self.bank.extra, non_blocking=True)
+                self.host_motion.copy_(self.motion.info, non_blocking=True)
             self._rows_downloaded.record(self._d2h_stream)
         return self.host_rows, self.host_counts
 
@@ -232,11 +275,12 @@ class DetectTrackPipeline:
         self._rows_downloaded.synchronize()
         self._post_done.synchronize()
         check_bank(self.host_stats, self.host_counts, self.bank.capacity, self.bank.max_out)
+        out = self.host_rows, self.host_counts
         if int(self.host_stats[:, 2].max()) + 2 * self.max_det > self.bank.capacity and self.bank.capacity < 65535:
             self.bank.grow(min(65535, 2 * self.bank.capacity))
             if not self._fixed_out:
-                self._alloc_host()
-        return self.host_rows, self.host_counts
+                self._regrow_host = True        # the next step_host reallocates: this step's host block stays valid until then
+        return out
 
 
 def check_frames(frames, shapes):

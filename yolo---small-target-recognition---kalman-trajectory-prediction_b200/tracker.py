@@ -66,6 +66,11 @@ class TrackerBank:
     def reset(self):
         _lib.check(self.lib.b2_tracker_reset(self._h, _lib.stream_ptr()))
 
+    def reset_streams(self, flags, stream=None):
+        """``reset()`` for the streams whose CUDA int32 ``flags`` [S] entry is non-zero, ordered on the stream (no synchronisation)."""
+        assert flags.is_cuda and flags.dtype.itemsize == 4 and flags.numel() == self.S
+        _lib.check(self.lib.b2_tracker_reset_streams(self._h, _lib.ptr(flags), _lib.stream_ptr(stream)))
+
     def grow(self, new_capacity):
         """Enlarge every stream's bank to ``new_capacity`` slots (state, ids and slot indices are kept; synchronises)."""
         _lib.check(self.lib.b2_tracker_grow(self._h, int(new_capacity), _lib.stream_ptr()))
@@ -89,10 +94,12 @@ class TrackerBank:
                                                  _lib.stream_ptr(stream)))
         return self.rows, self.counts
 
-    def stats_async(self, stream=None):
-        """[S][8] int64 device snapshot {created, terminated, active, long_term, recoveries, dropped, 0, 0}, stream-ordered."""
-        _lib.check(self.lib.b2_tracker_stats(self._h, _lib.ptr(self.stats_dev), _lib.stream_ptr(stream)))
-        return self.stats_dev
+    def stats_async(self, stream=None, out=None):
+        """[S][8] int64 device snapshot {created, terminated, active, long_term, recoveries, dropped, 0, 0} (mode 1: [6], [7] =
+        individual_resets, tracking_recoveries), stream-ordered, into ``out`` (default: an internal buffer)."""
+        out = self.stats_dev if out is None else out
+        _lib.check(self.lib.b2_tracker_stats(self._h, _lib.ptr(out), _lib.stream_ptr(stream)))
+        return out
 
     def predict_only(self, stream=None):
         """AircraftKalmanTracker.predict alone on every live track."""
@@ -339,6 +346,76 @@ class MotionCompensatedMultiTracker(EnhancedMultiTargetTracker):
         d["active_trackers"] = self._active
         d["motion_detector"] = dict(self.motion_detector.stats)
         return d
+
+
+MOTION_STAT_KEYS = ("total_detections", "motion_events", "reset_triggers", "avg_motion_magnitude", "global_motion_events", "global_resets")
+
+
+class GlobalMotionBank:
+    """:class:`GlobalMotionDetector` and the global-reset decision of :class:`MotionCompensatedMultiTracker` for S streams on the GPU
+    (csrc/motion.cu): per frame ``flow(frames)`` (gray pyramid, corners of the previous frame, pyramidal LK into this one; frames
+    only) then ``decide(det_counts)`` (the detector's vector and thresholds, ``_should_global_reset``).  ``decide`` returns device
+    tensors: flags int32 [S] (1 where the stream's tracks are to be dropped: ``TrackerBank.reset_streams``) and info float32 [S][8]
+    {magnitude, vx, vy, is_motion, should_reset, global_reset, corners, tracked corners}.  frame_shapes: one (h, w) or S of them;
+    frames are CUDA uint8 [S][h][w][3] or, for mixed shapes, packed by ``ops.pack_frames``."""
+
+    def __init__(self, n_streams, frame_shapes, device=None):
+        import torch
+
+        from . import ops
+
+        self.device = device or _lib.require_cuda()
+        self.lib = _lib.load()
+        self.S = int(n_streams)
+        shapes = [tuple(hw) for hw in frame_shapes] if hasattr(frame_shapes[0], "__len__") else [tuple(frame_shapes)] * self.S
+        if len(shapes) != self.S:
+            raise ValueError(f"frame_shapes lists {len(shapes)} shapes for {self.S} streams")
+        self.frame_shapes = [(int(h), int(w)) for h, w in shapes]
+        sh = np.ascontiguousarray(np.asarray(self.frame_shapes, np.int32))
+        self._h = C.c_void_p()
+        _lib.check(self.lib.b2_motion_create(self.S, sh.ctypes.data_as(C.c_void_p), C.byref(self._h)))
+        self.uniform = len(set(self.frame_shapes)) == 1
+        offs = (np.arange(self.S, dtype=np.int64) * (self.frame_shapes[0][0] * self.frame_shapes[0][1] * 3) if self.uniform
+                else ops.pack_layout(self.frame_shapes)[0])
+        self.offsets = torch.from_numpy(offs).to(self.device)
+        self.flags = torch.zeros((self.S,), dtype=torch.int32, device=self.device)
+        self.info = torch.zeros((self.S, 8), dtype=torch.float32, device=self.device)
+        self.stats_dev = torch.zeros((self.S, 8), dtype=torch.float64, device=self.device)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self.lib.b2_motion_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    def reset(self, stream=None):
+        """Forget every stream's previous frame and decision history."""
+        _lib.check(self.lib.b2_motion_reset(self._h, _lib.stream_ptr(stream)))
+
+    def flow(self, frames, offsets=None, stream=None):
+        """frames: CUDA uint8, [S][h][w][3] or the packed layout (``offsets``: CUDA int64 [S] byte offsets, default: ``ops.pack_layout``)."""
+        assert frames.is_cuda and frames.is_contiguous() and frames.dtype.itemsize == 1
+        offsets = self.offsets if offsets is None else offsets
+        _lib.check(self.lib.b2_motion_flow(self._h, _lib.ptr(frames), _lib.ptr(offsets), _lib.stream_ptr(stream)))
+
+    def decide(self, det_counts=None, tracker_stats=None, stream=None):
+        """det_counts: CUDA int32 [S] detections of this frame (None: 0); tracker_stats: ``TrackerBank.stats_async()`` before the
+        reset (feeds the individual-resets / recoveries base), or None.  Returns (flags, info) device tensors."""
+        _lib.check(self.lib.b2_motion_decide(self._h, _lib.ptr(det_counts), _lib.ptr(tracker_stats), _lib.ptr(self.flags), _lib.ptr(self.info),
+                                             _lib.stream_ptr(stream)))
+        return self.flags, self.info
+
+    def stats_async(self, stream=None):
+        """[S][8] float64 device snapshot {total_detections, motion_events, reset_triggers, avg_motion_magnitude, global_motion_events,
+        global_resets, individual-resets base, recoveries base}, stream-ordered."""
+        _lib.check(self.lib.b2_motion_stats(self._h, _lib.ptr(self.stats_dev), _lib.stream_ptr(stream)))
+        return self.stats_dev
+
+    def stats(self):
+        """Per stream: the detector's ``stats`` dict plus the tracker's global_motion_events / global_resets (synchronises)."""
+        st = self.stats_async().cpu().numpy()
+        return [{k: (float(v) if k == "avg_motion_magnitude" else int(v)) for k, v in zip(MOTION_STAT_KEYS, row)} for row in st]
 
 
 class GlobalMotionDetector:
